@@ -31,6 +31,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 
 METRIC = "blurry_views_per_s_fwd_bwd"
 UNIT = "views/s"
@@ -398,20 +399,40 @@ def cpu_baseline(bench_config):
                                   "backward incl. the pose chain, in %.1f s" % t_c1}}
 
 
+PARAM_NAMES = ["xyz", "features_dc", "features_rest", "scaling", "rotation", "opacity", "ctrl_trans", "ctrl_rot", "nu"]
+DUMP_MAX_ELEMENTS = 1 << 20     # per array: 4 MB of float32, so that the nine gradients and the loss stay under 64 MB
+
+
+def dump_outputs(w, loss, out_dir):
+    """Writes what one step hands its caller -- the loss and the gradient of every parameter -- as <name>.npy (float32;
+    the loss float64).  An array of more than DUMP_MAX_ELEMENTS elements is replaced by the elements at a fixed set of
+    flat indices (seeded by its size, sorted), so two builds dumped with the same arguments compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([float(loss.item())], dtype=np.float64))
+    params = w["gaussians"].parameters() + w["cmm"].parameters()
+    for name, p in zip(PARAM_NAMES, params):
+        g = p.grad.detach().reshape(-1).float()
+        if g.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randperm(g.numel(), generator=torch.Generator().manual_seed(g.numel()))[:DUMP_MAX_ELEMENTS]
+            g = g[idx.sort().values.to(g.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), g.cpu().numpy())
+
+
 def time_steps(step, gt_dev, steps, world, device):
     """`steps` steps between two CUDA events on the current stream; ms per step, max over ranks."""
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier(world)
     e0.record()
     for _ in range(steps):
-        step(gt_dev)
+        loss = step(gt_dev)
     e1.record()
     barrier(world)
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=device)
     if world > 1:
         import torch.distributed as dist
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    return float(t.item()) / steps
+    return float(t.item()) / steps, loss
 
 
 def other_config(name, rank, world, device, steps=3, warmup=3):
@@ -431,7 +452,7 @@ def other_config(name, rank, world, device, steps=3, warmup=3):
     gt = w["gt_host"].to(device)
     for _ in range(warmup):
         step(gt)
-    ms = time_steps(step, gt, steps, world, device)
+    ms = time_steps(step, gt, steps, world, device)[0]
     loss = float(step(gt).item())
     P, W, H, F = w["P"], w["W"], w["H"], w["F"]
     mode_str = getattr(step, "mode", "kernel by kernel")
@@ -461,7 +482,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch the step kernel by kernel instead of replaying a CUDA graph")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the c3 / c4 lines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and parameter gradients to DIR/<name>.npy "
+                         "(a fixed sample of 2^20 elements of a larger gradient)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE JSON line: everything else any library prints while the run lasts (NCCL's version
     # banner, torch warnings) goes to stderr at the file-descriptor level; `emit` writes to the real stdout.
@@ -504,7 +530,7 @@ def main():
         lib.dgs_launch_count(1)
     sampler = ClockSampler(local)
     sampler.start()
-    ms_step = time_steps(step, gt_dev, args.steps, eff_world, device)
+    ms_step, last_loss = time_steps(step, gt_dev, args.steps, eff_world, device)
     sampler.stop_flag = True
     sampler.join()
     launches = None
@@ -513,6 +539,8 @@ def main():
         if step.graph is not None:     # kernels inside a replayed graph are not seen by the launch counter
             step.graph.check()
             launches += step.graph.launches_per_replay * args.steps
+    if args.dump_outputs and rank == 0:   # after check(): a replay past the graph's capacity is redone there
+        dump_outputs(w, step.graph.loss if getattr(step, "graph", None) is not None else last_loss, args.dump_outputs)
     views_per_step = 1 if sharded else eff_world
     value = views_per_step * 1000.0 / ms_step
 

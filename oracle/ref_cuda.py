@@ -36,8 +36,6 @@ def load():
         lib.ref_knn.restype = None
         lib.ref_knn.argtypes = [i, p, p]
         lib.ref_sync.restype = i
-        lib.truth_blend_backward.restype = None
-        lib.truth_blend_backward.argtypes = [i, i] + [p] * 8 + [f] + [p] * 7
         _lib = lib
     return _lib
 
@@ -143,21 +141,32 @@ def knn(points):
     return out
 
 
-def truth_blend_backward(fw, bg, W, H, dL_dpix, dL_dpixdepth, z_far=100.0):
-    """Float64 evaluation of the tile-blend backward (oracle/truth_bwd.cu) on the forward state `fw` of a
-    reference run: same blend decisions as the float forward, float64 values and sums. Returns the tuple
+TRUTH_LIB_PATH = os.path.join(HERE, "_build", "libtruth_bwd.so")
+_truth = None
+
+
+def truth_blend_backward(W, H, ranges, point_list, means2D, conic_opacity, rgb, depths, n_contrib, bg, dL_dpix,
+                         dL_dpixdepth, z_far=100.0):
+    """Float64 evaluation of the tile-blend backward (oracle/truth_bwd.cu, built by `make -C oracle truth`) on the
+    forward state of one view: ranges [tiles, 2] and point_list of that view's tile lists, the per-Gaussian means2D,
+    conic_opacity, rgb and depths, the per-pixel n_contrib (the decoded GeometryState / BinningState / ImageState
+    arrays).  Same blend decisions as the float forward, float64 values and sums. Returns the tuple
     rn.preprocess_backward takes: (dL_dmean2D [P,2] w.r.t. NDC, dL_dconic [P,3], dL_dopacity [P], dL_dcolor [P,3],
     dL_ddepth [P]) as float64 CUDA tensors."""
-    lib = load()
+    global _truth
+    if _truth is None:
+        lib = C.CDLL(TRUTH_LIB_PATH)
+        lib.truth_blend_backward.restype = None
+        lib.truth_blend_backward.argtypes = [C.c_int, C.c_int] + [C.c_void_p] * 8 + [C.c_float] + [C.c_void_p] * 7
+        _truth = lib
     dev = bg.device
-    P = fw["radii"].shape[0]
+    P = means2D.shape[0]
     z = lambda *s: torch.zeros(s, dtype=torch.float64, device=dev)
     dmean, dconic, dop, dcol, ddep = z(P, 2), z(P, 3), z(P), z(P, 3), z(P)
-    g, b, im = fw["geom"], fw["binning"], fw["image"]
+    args = [t.contiguous() for t in (ranges, point_list, means2D, conic_opacity, rgb, depths, n_contrib, bg)]
+    grads = [t.contiguous() for t in (dL_dpix, dL_dpixdepth)]
     torch.cuda.synchronize(dev)
-    lib.truth_blend_backward(W, H, _ptr(im["ranges"]), _ptr(b["point_list"]), _ptr(g["means2D"]),
-                             _ptr(g["conic_opacity"]), _ptr(g["rgb"]), _ptr(g["depths"]), _ptr(im["n_contrib"]),
-                             _ptr(bg), z_far, _ptr(dL_dpix), _ptr(dL_dpixdepth), _ptr(dmean), _ptr(dconic),
-                             _ptr(dop), _ptr(dcol), _ptr(ddep))
-    lib.ref_sync()
+    _truth.truth_blend_backward(W, H, *[_ptr(t) for t in args], z_far, *[_ptr(t) for t in grads], _ptr(dmean),
+                                _ptr(dconic), _ptr(dop), _ptr(dcol), _ptr(ddep))   # legacy default stream
+    torch.cuda.synchronize(dev)
     return dmean, dconic, dop, dcol, ddep

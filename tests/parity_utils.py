@@ -1,10 +1,12 @@
-"""Shared helpers for the GPU parity tests: run libdgs_b200 (through the package's C-ABI binding) and
-the reference's own CUDA rasterizer (oracle/_ref, test infrastructure) on identical device buffers
-and compare every intermediate the reference defines."""
+"""Shared helpers for the GPU parity tests: run libdgs_b200 (through the package's C-ABI binding), decode
+every intermediate the reference defines, and compare them with the reference's outputs stored in
+tests/golden/parity.npz."""
 import ctypes as C
+import hashlib
 import os
 import sys
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -92,6 +94,118 @@ def ours_backward(cam, scene, bg, view, proj, campos, fw, dL_dpix, dL_ddepth, sh
                                fw["radii"], fw["geom"], fw["binning"], fw["img"], dL_dpix, dL_ddepth, True,
                                want_stats=True)
     return dict(zip(names + ["densify_stats"], out))
+
+
+GOLDEN = os.path.join(ROOT, "tests", "golden", "parity.npz")
+WHOLE = 384       # float tensors up to this size are stored whole
+SAMPLE = 320      # larger ones: this many elements at seeded random positions ...
+TAIL = 64         # ... and their last elements (the last Gaussians; the last rows of the last image)
+_STORE = None
+
+
+def _sample_index(n):
+    if n <= WHOLE:
+        return torch.arange(n)
+    idx = torch.randint(0, n - TAIL, (SAMPLE,), generator=torch.Generator().manual_seed(n))
+    return torch.cat([idx.unique(), torch.arange(n - TAIL, n)])
+
+
+class Golden:
+    """Stored outputs of one test case, in tests/golden/parity.npz as three arrays per case: <case>.names (the fields),
+    <case>.exact (per bit-exact field: the SHA-256 digest of its bytes, then its shape as four int64) and
+    <case>.sample (per float field, concatenated: the tensor whole up to WHOLE elements, otherwise the elements at
+    _sample_index, each followed by the tensor's max |x|).
+
+    The vectors were recorded from this library's kernels as they were when the parity suite last ran against the
+    reference's own CUDA rasterizer, simple-knn and extension module on a B200, with every list bit-identical and every
+    image and gradient within the bars the tests apply (profiles/r2_final_gpu_tests.log): they stand in for the
+    reference's outputs, which need the reference's sources to produce.
+    With DGS_RECORD_GOLDEN=<dir> set, the tests write one <case>.npz per case to <dir> instead of comparing;
+    pack(<dir>) merges them into tests/golden/parity.npz."""
+
+    def __init__(self, case):
+        global _STORE
+        self.case = case
+        self.record_dir = os.environ.get("DGS_RECORD_GOLDEN")
+        self.exacts, self.samples = {}, {}
+        if self.record_dir:
+            return
+        if _STORE is None:
+            with np.load(GOLDEN) as z:
+                _STORE = {k: z[k] for k in z.files}
+        names = list(_STORE[case + ".names"])
+        ex, sm = _STORE[case + ".exact"], _STORE[case + ".sample"]
+        off = 0
+        for name in names:
+            kind, key = name.split(":", 1)
+            if kind == "x":
+                self.exacts[key] = ex[len(self.exacts)]
+            else:
+                n = int(kind[1:])
+                self.samples[key] = sm[off:off + n + 1]
+                off += n + 1
+
+    def exact(self, key, t):
+        """t bit for bit."""
+        t = t.detach().contiguous().cpu()
+        assert t.dim() <= 4
+        shape = np.zeros(4, np.int64)
+        shape[:t.dim()] = t.shape
+        d = np.concatenate([np.frombuffer(hashlib.sha256(t.view(torch.uint8).numpy().tobytes()).digest(), np.uint8),
+                            shape.view(np.uint8)])
+        if self.record_dir:
+            self.exacts[key] = d
+        assert np.array_equal(self.exacts[key], d), (self.case, key, tuple(t.shape))
+
+    def sample(self, key, t):
+        """(this run's sample of t, the stored sample, the stored max |x| of the whole tensor), float64 on the CPU."""
+        t = t.detach().reshape(-1)
+        n = t.numel()
+        mine = t[_sample_index(n).to(t.device)].cpu()
+        if self.record_dir:
+            self.samples[key] = np.append(mine.float().numpy(), np.float32(t.abs().max().item() if n else 0.0))
+        stored = torch.from_numpy(self.samples[key]).double()
+        assert stored.numel() == mine.numel() + 1, (self.case, key)
+        return mine.double(), stored[:-1], float(stored[-1])
+
+    def abs_close(self, key, t, tol):
+        """max |t - stored| <= tol on the stored elements."""
+        a, b, _ = self.sample(key, t)
+        err = float((a - b).abs().max()) if a.numel() else 0.0
+        assert err <= tol, (self.case, key, err, tol)
+
+    def rel_close(self, key, t, tol):
+        """max |t - stored| / max |stored| <= tol (the stored elements' errors over the whole tensor's max)."""
+        a, b, m = self.sample(key, t)
+        err = float((a - b).abs().max()) / max(m, 1e-30) if a.numel() else 0.0
+        assert err <= tol, (self.case, key, err, tol)
+
+    def rel_err(self, key, t, floor_frac=1e-3):
+        """rel_err (below) of t against the stored elements."""
+        a, b, m = self.sample(key, t)
+        if m == 0:
+            return float((a - b).abs().max()) if a.numel() else 0.0
+        return float(((a - b).abs() / b.abs().clamp_min(floor_frac * m)).max())
+
+    def done(self):
+        if not self.record_dir:
+            return
+        names = ["x:" + k for k in self.exacts] + ["s%d:%s" % (len(v) - 1, k) for k, v in self.samples.items()]
+        ex = np.stack(list(self.exacts.values())) if self.exacts else np.zeros((0, 64), np.uint8)
+        sm = np.concatenate(list(self.samples.values())) if self.samples else np.zeros(0, np.float32)
+        os.makedirs(self.record_dir, exist_ok=True)
+        np.savez_compressed(os.path.join(self.record_dir, self.case + ".npz"), names=np.array(names), exact=ex,
+                            sample=sm.astype(np.float32))
+
+
+def pack(record_dir, out=GOLDEN):
+    """Merge the per-case files a recording run wrote into one archive."""
+    arrays = {}
+    for f in sorted(os.listdir(record_dir)):
+        with np.load(os.path.join(record_dir, f)) as z:
+            for k in z.files:
+                arrays[f[:-len(".npz")] + "." + k] = z[k]
+    np.savez_compressed(out, **arrays)
 
 
 def rel_err(a, b, floor_frac=1e-3):

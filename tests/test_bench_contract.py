@@ -5,6 +5,7 @@ import json
 import os
 import subprocess
 import sys
+import time
 
 import torch
 
@@ -38,9 +39,18 @@ def test_peaks_and_clock_sampler_degrade_gracefully():
     hbm, src = bench.measured_peaks()
     assert hbm > 1000 and isinstance(src, str)
     s = bench.ClockSampler(0)
-    s.run()                                               # no NVML / no GPU here: returns immediately
+    s.start()                                             # without NVML run() returns at once; with it, it samples
+    time.sleep(0.1)
+    s.stop_flag = True
+    s.join(timeout=10)
+    assert not s.is_alive()
     out = s.summary()
-    assert set(out) == {"sm_mhz", "sm_max_mhz", "reasons", "samples"} and out["reasons"] == []
+    assert set(out) == {"sm_mhz", "sm_max_mhz", "reasons", "samples"}
+    if s.nv is None:
+        assert out["reasons"] == [] and out["samples"] == 0
+    else:
+        assert out["samples"] >= 1 and set(out["reasons"]) <= {"sw_power_cap", "hw_slowdown", "hw_thermal_slowdown",
+                                                                "sw_thermal_slowdown", "hw_power_brake"}
     json.dumps(out)
 
 

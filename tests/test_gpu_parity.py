@@ -1,6 +1,7 @@
 """GPU parity tests (pytest -m gpu): libdgs_b200 through its C-ABI binding against
-  (1) the reference's own CUDA rasterizer / simple-knn (oracle/_ref, compiled from the reference sources),
-  (2) the committed golden vectors (tests/golden/, produced by (1) / by the reference's Python),
+  (1) the outputs of the reference's own CUDA rasterizer / simple-knn / extension module on the same inputs, stored
+      in tests/golden/parity.npz (tests.parity_utils.Golden),
+  (2) the committed golden vectors (tests/golden/, produced by the reference's CUDA extension and Python),
   (3) the CPU restatement (oracle/raster_np.py, oracle/pose_torch.py),
 and size-independent properties at BASELINE.json's full c2 size.
 
@@ -9,7 +10,6 @@ gradients <= 1e-3 relative (max-abs error over the tensor's max-abs; the referen
 give ~1e-4 run-to-run).
 """
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -17,11 +17,10 @@ import torch
 
 from tests import parity_utils as pu
 from deblurgs_b200 import _lib, synthetic
-from oracle import ref_cuda
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref not built")
+GAUSS = ["dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"]
 
 
 def relmax(a, b):
@@ -39,58 +38,49 @@ def test_native_library_is_the_thing_running():
     assert lib.dgs_launch_count(0) - before >= 5
 
 
-def _compare_forward(name, sh_degree=3, use_sigmoid=False, P=None, F=None, mutate=None):
+def _compare_forward(name, sh_degree=3, use_sigmoid=False, P=None, F=None, mutate=None, case=None):
+    """Every forward intermediate against the reference's (stored) outputs on the same inputs."""
     cam, scene, traj, bg, view, proj, campos = pu.make_inputs(name, sh_degree=3, P=P, F=F)
     if mutate is not None:
         mutate(scene, view, campos)
     P, F, W, H = scene.means3D.shape[0], view.shape[0], cam.width, cam.height
-    tiles = ((W + 15) // 16) * ((H + 15) // 16)
     fw = pu.ours_forward(cam, scene, bg, view, proj, campos, sh_degree=sh_degree, use_sigmoid=use_sigmoid)
     dec = pu.ours_decode(fw, P, F, W, H)
     tb = dec["tile_bits"]
-    base, refs = 0, []
-    for s in range(F):
-        r = ref_cuda.forward(scene.means3D, scene.shs, None, scene.opacities, scene.scales, scene.rotations, None,
-                             view[s].contiguous(), proj[s].contiguous(), campos[s].contiguous(), bg, W, H,
-                             cam.tanfovx, cam.tanfovy, sh_degree, use_sigmoid=use_sigmoid)
-        refs.append(r)
-        vis = r["radii"] > 0
-        assert torch.equal(r["radii"], fw["radii"][s])
-        assert torch.equal(r["geom"]["tiles_touched"], dec["tiles_touched"][s])
-        assert torch.equal(r["geom"]["depths"].view(torch.int32)[vis], dec["depths"][s].view(torch.int32)[vis])
-        assert torch.equal(r["geom"]["means2D"].view(P, 2)[vis], dec["means2D"][s][vis])
-        assert torch.equal(r["geom"]["conic_opacity"].view(P, 4)[vis], dec["conic_opacity"][s][vis])
-        assert (r["geom"]["rgb"].view(P, 3)[vis] - dec["rgb"][s][vis]).abs().max() <= 1e-6
-        R = r["num_rendered"]
-        keys = dec["keys"][base:base + R]
-        assert torch.equal(keys & ((1 << (32 + tb)) - 1), r["binning"]["point_list_keys"])   # low bits = reference key
-        assert bool(((keys >> (32 + tb)) == s).all())                                           # high bits = sub-frame
-        assert torch.equal(dec["point_list"][base:base + R], r["binning"]["point_list"])
-        mine = dec["ranges"][s].clone()
-        nz = mine[:, 1] > mine[:, 0]
-        mine[nz] -= base
-        assert torch.equal(mine, r["image"]["ranges"][:2 * tiles].view(tiles, 2))
-        assert torch.equal(r["image"]["n_contrib"].view(H, W), dec["n_contrib"][s])
-        assert (r["image"]["accum_alpha"].view(H, W) - dec["final_T"][s]).abs().max() <= 1e-6
-        assert (r["color"] - fw["color"][s]).abs().max() <= 1e-4
-        # depth image: 1e-4 of its scale (z_far = 100 unless a test plants Gaussians further out; the blend weights
-        # alpha * T are shared between colour and depth here, so a term differs from the reference's by an ulp)
-        assert (r["depth"] - fw["depth"][s]).abs().max() <= 1e-4 * max(100.0, float(r["depth"].abs().max()))
-        base += R
-    assert base == fw["num_rendered"]
-    blur = torch.stack([r["color"] for r in refs]).mean(0)
-    assert (blur - fw["blur"]).abs().max() <= 1e-4
-    return cam, scene, bg, view, proj, campos, fw, refs
+    gd = pu.Golden(case or "fwd_%s_deg%d%s" % (name, sh_degree, "_sigmoid" if use_sigmoid else ""))
+    vis = fw["radii"] > 0
+    gd.exact("radii", fw["radii"])
+    gd.exact("tiles_touched", dec["tiles_touched"])
+    gd.exact("depths", dec["depths"].view(torch.int32)[vis])
+    gd.exact("means2D", dec["means2D"][vis])
+    gd.exact("conic_opacity", dec["conic_opacity"][vis])
+    gd.abs_close("rgb", dec["rgb"][vis], 1e-6)
+    counts = dec["tiles_touched"].long().sum(1)
+    assert int(counts.sum()) == fw["num_rendered"]
+    keys = dec["keys"]
+    sub = torch.repeat_interleave(torch.arange(F, device=keys.device), counts)
+    assert bool(((keys >> (32 + tb)) == sub).all())                                  # high bits = sub-frame
+    gd.exact("keys", keys & ((1 << (32 + tb)) - 1))                                # low bits = reference key
+    gd.exact("point_list", dec["point_list"])
+    gd.exact("ranges", dec["ranges"])
+    gd.exact("n_contrib", dec["n_contrib"])
+    gd.abs_close("final_T", dec["final_T"], 1e-6)
+    gd.abs_close("color", fw["color"], 1e-4)
+    # depth image: 1e-4 of its scale (z_far = 100 unless a test plants Gaussians further out; the blend weights
+    # alpha * T are shared between colour and depth here, so a term differs from the reference's by an ulp)
+    a, b, m = gd.sample("depth", fw["depth"])
+    assert (a - b).abs().max() <= 1e-4 * max(100.0, m)
+    gd.abs_close("blur", fw["blur"], 1e-4)
+    gd.done()
+    return cam, scene, bg, view, proj, campos, fw
 
 
-@needs_ref
 @pytest.mark.parametrize("name,deg,sig", [("tiny", 3, False), ("tiny", 0, False), ("tiny", 1, False), ("tiny", 2, False),
                                           ("tiny", 3, True), ("small", 3, False), ("c1", 3, False)])
 def test_forward_bit_exact_vs_reference_cuda(name, deg, sig):
     _compare_forward(name, sh_degree=deg, use_sigmoid=sig)
 
 
-@needs_ref
 @pytest.mark.parametrize("F,far", [(16, 2.0e9), (32, 5.0e4), (16, 1.0e3), (40, 30.0)])
 def test_depth_key_paths_give_the_reference_order(F, far):
     """The depth order is a segmented sort on the 32 raw depth bits (exact for any positive depth, any F).
@@ -104,63 +94,49 @@ def test_depth_key_paths_give_the_reference_order(F, far):
         scene.means3D[:k] = campos[0][None] + fwd[None] * far * jitter
         scene.scales[:k] = far * 0.01                          # ~7 px footprint at any distance
         scene.opacities[:k] = 0.8
-    _, scene, _, view, _, _, fw, refs = _compare_forward("tiny", F=F, mutate=plant)
+    _, scene, _, view, _, _, fw = _compare_forward("tiny", F=F, mutate=plant, case="fwd_depthkey_F%d_far%d" % (F, far))
     assert int((fw["radii"][0][:6] > 0).sum()) >= 1            # the planted Gaussians are actually rendered
 
 
-@needs_ref
 @pytest.mark.parametrize("name", ["small", "c1"])
 def test_backward_without_a_depth_gradient(name):
     """The blend backward has its own instantiation for "no gradient of the depth image" (the photometric losses:
     the entry's depth is not read, dL/dpix is three components).  Against the reference with a zero depth gradient,
     and against this library's own with-depth instantiation fed the same zeros."""
-    cam, scene, bg, view, proj, campos, fw, refs = _compare_forward(name)
+    cam, scene, bg, view, proj, campos, fw = _compare_forward(name)
     F, W, H = view.shape[0], cam.width, cam.height
     g = torch.Generator().manual_seed(11)
     dpix = (torch.randn(F, 3, H, W, generator=g) / (3 * H * W)).cuda()
     zeros = torch.zeros(F, 1, H, W).cuda()
     mine = pu.ours_backward(cam, scene, bg, view, proj, campos, fw, dpix, None)
     with_zeros = pu.ours_backward(cam, scene, bg, view, proj, campos, fw, dpix, zeros)
-    acc = None
-    for s in range(F):
-        b = ref_cuda.backward(refs[s], scene.means3D, scene.shs, None, scene.scales, scene.rotations, None,
-                              view[s].contiguous(), proj[s].contiguous(), campos[s].contiguous(), bg, W, H,
-                              cam.tanfovx, cam.tanfovy, 3, dpix[s].contiguous(), zeros[s].contiguous())
-        acc = {k: v.double().clone() for k, v in b.items()} if acc is None else {k: acc[k] + v.double() for k, v in b.items()}
-    for k in ["dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"]:
-        assert relmax(mine[k], acc[k]) <= 1e-3, k
+    gd = pu.Golden("bwd_nodepth_%s" % name)       # the reference's gradients, summed over the sub-frames
+    for k in GAUSS:
+        gd.rel_close(k, mine[k], 1e-3)
         assert relmax(mine[k], with_zeros[k]) <= 1e-5, k        # same sums; only the order of the float REDs differs
     for k in ["dL_dviewmatrix", "dL_dprojmatrix", "dL_dmeans2D"]:
         assert relmax(mine[k], with_zeros[k]) <= 1e-5, k
+    gd.done()
 
 
-@needs_ref
 @pytest.mark.parametrize("name,sig", [("tiny", False), ("tiny", True), ("small", False), ("c1", False)])
 def test_backward_vs_reference_cuda(name, sig):
-    cam, scene, bg, view, proj, campos, fw, refs = _compare_forward(name, use_sigmoid=sig)
+    cam, scene, bg, view, proj, campos, fw = _compare_forward(name, use_sigmoid=sig)
     F, W, H = view.shape[0], cam.width, cam.height
     g = torch.Generator().manual_seed(7)
     dpix = (torch.randn(F, 3, H, W, generator=g) / (3 * H * W)).cuda()
     ddep = (torch.randn(F, 1, H, W, generator=g) / (H * W) * 0.1).cuda()
     mine = pu.ours_backward(cam, scene, bg, view, proj, campos, fw, dpix, ddep, use_sigmoid=sig)
-    acc, per = None, []
-    for s in range(F):
-        b = ref_cuda.backward(refs[s], scene.means3D, scene.shs, None, scene.scales, scene.rotations, None,
-                              view[s].contiguous(), proj[s].contiguous(), campos[s].contiguous(), bg, W, H,
-                              cam.tanfovx, cam.tanfovy, 3, dpix[s].contiguous(), ddep[s].contiguous(), use_sigmoid=sig)
-        per.append(b)
-        acc = {k: v.double().clone() for k, v in b.items()} if acc is None else {k: acc[k] + v.double() for k, v in b.items()}
-    for k in ["dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"]:
-        assert relmax(mine[k], acc[k]) <= 1e-3, k
-    assert relmax(mine["dL_dviewmatrix"], torch.stack([b["dL_dviewmatrix"] for b in per])) <= 1e-3
-    assert relmax(mine["dL_dprojmatrix"], torch.stack([b["dL_dprojmatrix"] for b in per])) <= 1e-3
-    assert relmax(mine["dL_dmeans2D"], torch.stack([b["dL_dmeans2D"] for b in per])) <= 1e-3
+    # the reference's gradients: Gaussian ones summed over the sub-frames, matrix / screen-space ones per sub-frame
+    gd = pu.Golden("bwd_%s%s" % (name, "_sigmoid" if sig else ""))
+    for k in GAUSS + ["dL_dviewmatrix", "dL_dprojmatrix", "dL_dmeans2D"]:
+        gd.rel_close(k, mine[k], 1e-3)
+    gd.done()
     # culled Gaussians get exactly zero gradient (backward.cu:158,393)
     dead = (fw["radii"] <= 0).all(dim=0)
     assert float(mine["dL_dmeans3D"][dead].abs().max() if dead.any() else 0.0) == 0.0
 
 
-@needs_ref
 def test_precomputed_colors_and_covariance_and_scale_modifier():
     cam, scene, traj, bg, view, proj, campos = pu.make_inputs("tiny")
     P, F, W, H = scene.means3D.shape[0], view.shape[0], cam.width, cam.height
@@ -180,29 +156,19 @@ def test_precomputed_colors_and_covariance_and_scale_modifier():
     for kw in [dict(colors_precomp=colors), dict(cov3D_precomp=cov), dict(scale_modifier=0.7)]:
         fw = pu.ours_forward(cam, scene, bg, view, proj, campos, **kw)
         mine = pu.ours_backward(cam, scene, bg, view, proj, campos, fw, dpix, ddep, **kw)
-        cp, cv, mod = kw.get("colors_precomp"), kw.get("cov3D_precomp"), kw.get("scale_modifier", 1.0)
-        acc = None
-        for s in range(F):
-            r = ref_cuda.forward(scene.means3D, None if cp is not None else scene.shs, cp, scene.opacities,
-                                 None if cv is not None else scene.scales, None if cv is not None else scene.rotations,
-                                 cv, view[s].contiguous(), proj[s].contiguous(), campos[s].contiguous(), bg, W, H,
-                                 cam.tanfovx, cam.tanfovy, 3, scale_modifier=mod)
-            assert torch.equal(r["radii"], fw["radii"][s])
-            assert (r["color"] - fw["color"][s]).abs().max() <= 1e-4
-            b = ref_cuda.backward(r, scene.means3D, None if cp is not None else scene.shs, cp,
-                                  None if cv is not None else scene.scales, None if cv is not None else scene.rotations,
-                                  cv, view[s].contiguous(), proj[s].contiguous(), campos[s].contiguous(), bg, W, H,
-                                  cam.tanfovx, cam.tanfovy, 3, dpix[s].contiguous(), ddep[s].contiguous(),
-                                  scale_modifier=mod)
-            acc = {k: v.double().clone() for k, v in b.items()} if acc is None else {k: acc[k] + v.double() for k, v in b.items()}
-        assert relmax(mine["dL_dmeans3D"], acc["dL_dmeans3D"]) <= 1e-3
+        cp, cv = kw.get("colors_precomp"), kw.get("cov3D_precomp")
+        gd = pu.Golden("precomp_" + next(iter(kw)))
+        gd.exact("radii", fw["radii"])
+        gd.abs_close("color", fw["color"], 1e-4)
+        gd.rel_close("dL_dmeans3D", mine["dL_dmeans3D"], 1e-3)
         if cp is not None:
-            assert relmax(mine["dL_dcolors"], acc["dL_dcolors"]) <= 1e-3
+            gd.rel_close("dL_dcolors", mine["dL_dcolors"], 1e-3)
         if cv is not None:
-            assert relmax(mine["dL_dcov3D"], acc["dL_dcov3D"]) <= 1e-3
+            gd.rel_close("dL_dcov3D", mine["dL_dcov3D"], 1e-3)
         else:
-            assert relmax(mine["dL_dscales"], acc["dL_dscales"]) <= 1e-3
-            assert relmax(mine["dL_drotations"], acc["dL_drotations"]) <= 1e-3
+            gd.rel_close("dL_dscales", mine["dL_dscales"], 1e-3)
+            gd.rel_close("dL_drotations", mine["dL_drotations"], 1e-3)
+        gd.done()
 
 
 @pytest.mark.parametrize("tag,sig", [("tiny", False), ("tiny_sigmoid", True)])
@@ -293,11 +259,10 @@ def test_edge_cases():
     v1, p1, c1 = view[:1].contiguous(), proj[:1].contiguous(), campos[:1].contiguous()
     fw = pu.ours_forward(cam2, sc2, bg, v1, p1, c1)
     assert fw["color"].shape == (1, 3, 37, 75) and torch.isfinite(fw["color"]).all()
-    if ref_cuda.available():
-        r = ref_cuda.forward(sc2.means3D, sc2.shs, None, sc2.opacities, sc2.scales, sc2.rotations, None,
-                             v1[0].contiguous(), p1[0].contiguous(), c1[0].contiguous(), bg, 75, 37, cam2.tanfovx,
-                             cam2.tanfovy, 3)
-        assert torch.equal(r["radii"], fw["radii"][0]) and (r["color"] - fw["color"][0]).abs().max() <= 1e-4
+    gd = pu.Golden("edge_75x37")
+    gd.exact("radii", fw["radii"][0])
+    gd.abs_close("color", fw["color"][0], 1e-4)
+    gd.done()
 
 
 def test_batching_invariance_and_determinism():
@@ -350,25 +315,23 @@ def test_pose_kernel_vs_reference_python_golden(tag):
     assert relmax(nu_p.grad, c["g_nu_param"]) <= 1e-3
 
 
-@needs_ref
 @pytest.mark.parametrize("P", [5, 1000, 50_000, 2_000_000])
 def test_knn_matches_reference(P, capsys):
     from deblurgs_b200 import distCUDA2
     g = torch.Generator().manual_seed(P)
     pts = (torch.randn(P, 3, generator=g) * torch.tensor([3.0, 1.0, 0.3])).cuda()
     mine = distCUDA2(pts)
-    ref = ref_cuda.knn(pts)
-    assert torch.equal(mine, ref)
-    if P >= 1_000_000:      # post-densification scale: both searches timed (the coarse box level keeps ours near-linear)
-        def timed(fn):
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(); fn(pts); e1.record()
-            torch.cuda.synchronize()
-            return e0.elapsed_time(e1)
-        t_mine, t_ref = timed(distCUDA2), timed(ref_cuda.knn)
+    gd = pu.Golden("knn_%d" % P)
+    gd.exact("mean_dist2", mine)        # the reference's simple-knn result, bit for bit
+    gd.done()
+    if P >= 1_000_000:      # post-densification scale: timed (the coarse box level keeps the search near-linear)
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(); distCUDA2(pts); e1.record()
+        torch.cuda.synchronize()
+        t_mine = e0.elapsed_time(e1)
         with capsys.disabled():
-            print("\n  simple-knn at P = %d: library %.1f ms, reference %.1f ms" % (P, t_mine, t_ref))
+            print("\n  simple-knn at P = %d: library %.1f ms" % (P, t_mine))
         assert t_mine < 2000.0
     if P <= 1000:
         d = torch.cdist(pts.double(), pts.double()) ** 2
@@ -378,33 +341,30 @@ def test_knn_matches_reference(P, capsys):
 
 
 def test_drop_in_module_against_reference_extension():
-    """GaussianRasterizer (single view, autograd) against the reference's installed extension, if present."""
-    ref_dir = os.path.join(pu.ROOT, "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref_dir, "diff_gaussian_rasterization")):
-        pytest.skip("baseline/_ref not installed")
-    sys.path.insert(0, ref_dir)
-    import diff_gaussian_rasterization as ref_mod
+    """GaussianRasterizer (single view, autograd) against the reference's extension module (its stored outputs)."""
     import deblurgs_b200 as dg
     cam, scene, traj, bg, view, proj, campos = pu.make_inputs("tiny")
     W, H = cam.width, cam.height
     g = torch.Generator().manual_seed(1)
     wimg, wdep = torch.randn(3, H, W, generator=g).cuda(), torch.randn(1, H, W, generator=g).cuda() * 0.01
-    outs = []
-    for mod in (dg, ref_mod):
-        leaves = [t.clone().requires_grad_(True) for t in (scene.means3D, scene.shs, scene.opacities, scene.scales,
-                                                           scene.rotations, view[1], proj[1])]
-        m3, sh, op, sc, ro, vm, pm = leaves
-        m2 = torch.zeros_like(m3, requires_grad=True)
-        rs = mod.GaussianRasterizationSettings(H, W, cam.tanfovx, cam.tanfovy, bg, 1.0, 0.2, 100.0, False, 3,
-                                               campos[1], False, False)
-        img, dep, radii = mod.GaussianRasterizer(rs)(means3D=m3, means2D=m2, shs=sh, opacities=op, scales=sc,
-                                                     rotations=ro, viewmatrix=vm, projmatrix=pm)
-        ((img * wimg).sum() + (dep * wdep).sum()).backward()
-        outs.append((img.detach(), dep.detach(), radii, [t.grad for t in leaves] + [m2.grad]))
-    (i0, d0, r0, g0), (i1, d1, r1, g1) = outs
-    assert torch.equal(r0, r1) and (i0 - i1).abs().max() <= 1e-4 and (d0 - d1).abs().max() <= 1e-2
-    for a, b in zip(g0, g1):
-        assert a.shape == b.shape and relmax(a, b) <= 1e-3
+    leaves = [t.clone().requires_grad_(True) for t in (scene.means3D, scene.shs, scene.opacities, scene.scales,
+                                                       scene.rotations, view[1], proj[1])]
+    m3, sh, op, sc, ro, vm, pm = leaves
+    m2 = torch.zeros_like(m3, requires_grad=True)
+    rs = dg.GaussianRasterizationSettings(H, W, cam.tanfovx, cam.tanfovy, bg, 1.0, 0.2, 100.0, False, 3,
+                                          campos[1], False, False)
+    img, dep, radii = dg.GaussianRasterizer(rs)(means3D=m3, means2D=m2, shs=sh, opacities=op, scales=sc,
+                                                rotations=ro, viewmatrix=vm, projmatrix=pm)
+    ((img * wimg).sum() + (dep * wdep).sum()).backward()
+    gd = pu.Golden("dropin_tiny")
+    gd.exact("radii", radii)
+    gd.abs_close("image", img, 1e-4)
+    gd.abs_close("depth", dep, 1e-2)
+    grads = [t.grad for t in leaves] + [m2.grad]
+    for k, a in zip(["means3D", "shs", "opacities", "scales", "rotations", "viewmatrix", "projmatrix", "means2D"], grads):
+        gd.exact(k + "_shape", torch.tensor(a.shape))
+        gd.rel_close(k, a, 1e-3)
+    gd.done()
 
 
 def test_full_size_properties_c2():
