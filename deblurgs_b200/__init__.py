@@ -12,9 +12,9 @@ from .rasterizer import (GaussianRasterizationSettings, GaussianRasterizer, rast
 from .renderer import render, render_blurry
 from .pose import bezier_se3_poses
 from .knn import distCUDA2
-from .loss import blur_photometric_loss, hinge_l2, training_loss, tv_loss
+from .loss import blur_photometric_loss, hinge_l2, psnr, ssim, training_loss, tv_loss
 from .params import FusedAdam, activate_gaussians
 
 __all__ = ["GaussianRasterizationSettings", "GaussianRasterizer", "rasterize_gaussians", "rasterize_blurry",
            "render", "render_blurry", "bezier_se3_poses", "distCUDA2", "blur_photometric_loss", "tv_loss", "hinge_l2",
-           "training_loss", "FusedAdam", "activate_gaussians"]
+           "training_loss", "ssim", "psnr", "FusedAdam", "activate_gaussians"]

@@ -65,6 +65,9 @@ SIGNATURES = {
     "dgs_tv_loss_backward": (_i, [_i64, _i, _i, _p, _p, _p, _p]),
     "dgs_hinge_l2_forward": (_i, [_i64, _p, _p, _p, _p]),
     "dgs_hinge_l2_backward": (_i, [_i64, _p, _p, _p, _p]),
+    "dgs_ssim_scratch_bytes": (C.c_size_t, [_i, _i, _i, _i]),
+    "dgs_ssim_forward": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _p]),
+    "dgs_ssim_backward": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p]),
     "dgs_activate_forward": (_i, [_i, _i, _p, _p, _p, _p, _p, _f, _i, _p, _p, _p, _p, _p]),
     "dgs_activate_backward": (_i, [_i, _i, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "dgs_adam_step": (_i, [_i, _p, _p, _p, _p, C.POINTER(_i64), C.POINTER(C.c_double), C.POINTER(_i64),

@@ -10,13 +10,14 @@ and is looked at after the caller's own synchronisation (reading the loss).  If 
 step is re-captured with a larger one and replayed: results are always complete.
 
 Reference semantics: one iteration of train.py:121-163 for one image, without the optimizer step
-(`CameraMotionModule.query` + `l1_loss` (+ lambda_t_smooth * batchwise_smoothness_loss) + `loss.backward()`).
+(`CameraMotionModule.query` + `l1_loss` (+ lambda_t_smooth * batchwise_smoothness_loss) + `loss.backward()`); with
+lambda_dssim > 0 the L1 term is the 3DGS mix (1 - lambda_dssim) * L1 + lambda_dssim * (1 - SSIM).
 """
 import torch
 
 from . import _lib
 from . import rasterizer as rz
-from .loss import blur_photometric_loss
+from .loss import photometric_loss
 
 
 class BlurryViewGraph:
@@ -29,8 +30,10 @@ class BlurryViewGraph:
     `parameters` (default: the Gaussians' and the trajectory's) get their .grad from the captured backward."""
 
     def __init__(self, cmm, cam_idx, background, gt_shape, lambda_t_smooth=0.0, parameters=None, pre_backward=None,
-                 caller_owned_grads=(), capacity_margin=1.25, post_backward=None, render_fn=None):
+                 caller_owned_grads=(), capacity_margin=1.25, post_backward=None, render_fn=None,
+                 lambda_dssim=0.0):
         self.cmm, self.cam_idx, self.bg, self.lam = cmm, cam_idx, background, float(lambda_t_smooth)
+        self.lam_dssim = float(lambda_dssim)      # > 0: the D-SSIM term of loss.photometric_loss inside the graph
         dev = cmm.gaussians.get_xyz.device
         self.device = dev
         self.params = list(parameters) if parameters is not None else cmm.gaussians.parameters() + cmm.parameters()
@@ -59,7 +62,7 @@ class BlurryViewGraph:
             out = {"blurred": blurred, "subframes": subframes, "batched": pkg}
         else:
             out = self.cmm.query(self.cam_idx, "all", background=self.bg)
-        loss = blur_photometric_loss(out["blurred"], out["subframes"], self.gt, self.lam)
+        loss = photometric_loss(out["blurred"], out["subframes"], self.gt, self.lam, self.lam_dssim)
         loss.backward()
         if self.post_backward is not None:
             self.post_backward()

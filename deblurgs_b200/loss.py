@@ -1,7 +1,8 @@
 """Loss block of the blurry-view training step (reference: train.py:147-163, utils/loss_utils.py):
 `blur_photometric_loss` = l1_loss(blurred, gt) + lambda_t_smooth * batchwise_smoothness_loss(subframes), forward and
 backward in one kernel each; `tv_loss` (depth smoothness) and `hinge_l2` (opacity range penalty), one kernel each way;
-`training_loss` = the reference's weighted sum of the four."""
+`training_loss` = the reference's weighted sum of the four; `ssim` (one tile kernel each way, dgs_ssim.cu) for the
+3DGS D-SSIM term and for evaluation, `psnr` (utils/image_utils.py)."""
 import ctypes as C
 
 import torch
@@ -126,6 +127,67 @@ class _Hinge(torch.autograd.Function):
         return dx
 
 
+class _SSIM(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, img1, img2, size_average):
+        lib = _lib.load()
+        x = img1.detach().float().contiguous()
+        y = img2.detach().float().contiguous()
+        N, Cc, H, W = (1,) + tuple(x.shape) if x.dim() == 3 else tuple(x.shape)
+        out = torch.empty(1 + N, dtype=torch.float32, device=x.device)
+        nbytes = int(lib.dgs_ssim_scratch_bytes(N, Cc, H, W))
+        scratch = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=x.device)
+        # dS/dmu1, dS/dsigma1^2, dS/dsigma12 per pixel: only when img1 wants a gradient
+        maps = torch.empty((3,) + tuple(x.shape), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
+        with torch.cuda.device(x.device):
+            _lib.check(lib.dgs_ssim_forward(N, Cc, H, W, _lib.ptr(x), _lib.ptr(y), _lib.ptr(out), _lib.ptr(scratch),
+                                            _lib.ptr(maps), _st(x)), "dgs_ssim_forward")
+        if maps is not None:
+            ctx.save_for_backward(x, y, maps)
+        ctx.dims, ctx.size_average, ctx.shape = (N, Cc, H, W), size_average, img1.shape
+        return out[0] if size_average else out[1:]
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        lib = _lib.load()
+        x, y, maps = ctx.saved_tensors
+        N, Cc, H, W = ctx.dims
+        go = grad_out.detach().float().contiguous().reshape(-1)
+        dx = torch.empty_like(x)
+        with torch.cuda.device(x.device):
+            _lib.check(lib.dgs_ssim_backward(N, Cc, H, W, _lib.ptr(x), _lib.ptr(y), _lib.ptr(maps), _lib.ptr(go),
+                                             0 if ctx.size_average else 1, _lib.ptr(dx), _st(x)), "dgs_ssim_backward")
+        return dx.view(ctx.shape), None, None
+
+
+def ssim(img1, img2, window_size=11, size_average=True):
+    """utils/loss_utils.py `ssim` (3DGS): SSIM of [C,H,W] or [N,C,H,W] images with an 11x11 Gaussian window
+    (sigma 1.5, zero padding).  size_average=True: the mean over every pixel and channel (0-dim tensor); False: one
+    mean per image ([N], 4-D input only).  Differentiable in img1; img2 is a constant target."""
+    if img1.shape != img2.shape or img1.dim() not in (3, 4):
+        raise _lib.DgsError("ssim: img1 and img2 must have the same [C,H,W] or [N,C,H,W] shape, got %s and %s"
+                            % (tuple(img1.shape), tuple(img2.shape)))
+    if img1.numel() == 0:
+        raise _lib.DgsError("ssim: empty input %s" % (tuple(img1.shape),))
+    if window_size != 11:
+        raise _lib.DgsError("ssim: only window_size=11 is implemented")
+    if not size_average and img1.dim() != 4:
+        raise _lib.DgsError("ssim: size_average=False needs [N,C,H,W] input (one mean per image)")
+    if img2.requires_grad:
+        raise _lib.DgsError("ssim: img2 is treated as a constant target and gets no gradient; pass img2.detach()")
+    if not (img1.is_cuda and img2.is_cuda):
+        raise _lib.DgsError("ssim: CUDA tensors required (libdgs_b200 has no CPU path)")
+    if img1.device != img2.device:
+        raise _lib.DgsError("ssim: img1 and img2 are on different devices")
+    return _SSIM.apply(img1, img2, bool(size_average))
+
+
+def psnr(img1, img2):
+    """utils/image_utils.py `psnr`: 20 log10(1 / sqrt(mse)) per leading index, shape [N, 1]."""
+    mse = ((img1 - img2) ** 2).reshape(img1.shape[0], -1).mean(1, keepdim=True)
+    return 20 * torch.log10(1.0 / torch.sqrt(mse))
+
+
 def tv_loss(x):
     """utils/loss_utils.py:66-78 on a [B,C,H,W] tensor: l2 of the vertical + l2 of the horizontal neighbour differences."""
     return _TV.apply(x)
@@ -136,12 +198,26 @@ def hinge_l2(x):
     return _Hinge.apply(x)
 
 
+def photometric_loss(blurred, subframes, gt, lambda_t_smooth=0.0, lambda_dssim=0.0):
+    """Ll1 + lambda_t_smooth * L_t_smooth; with lambda_dssim > 0 the L1 term becomes the 3DGS D-SSIM mix
+    (1 - lambda_dssim) * Ll1 + lambda_dssim * (1 - ssim(blurred, gt)).  lambda_dssim == 0 runs no SSIM kernel."""
+    lam = float(lambda_dssim)
+    if lam == 0.0:
+        return blur_photometric_loss(blurred, subframes, gt, lambda_t_smooth)
+    if not 0.0 < lam < 1.0:
+        raise _lib.DgsError("lambda_dssim must lie in [0, 1), got %r" % (lambda_dssim,))
+    # (1 - lam) * (Ll1 + lambda_t / (1 - lam) * L_t_smooth): the fused L1 kernel keeps the smoothness weight unchanged
+    l1 = blur_photometric_loss(blurred, subframes, gt, float(lambda_t_smooth) / (1.0 - lam))
+    return (1.0 - lam) * l1 + lam * (1.0 - ssim(blurred, gt.detach()))
+
+
 def training_loss(blurred, subframes, gt, depths=None, opacity=None, lambda_t_smooth=0.0, lambda_depth_tv=0.0,
-                  lambda_hinge=0.0):
+                  lambda_hinge=0.0, lambda_dssim=0.0):
     """The reference's loss (train.py:147-163): Ll1 + lambda_t_smooth * L_t_smooth + lambda_depth_tv * L_depth_tv +
     lambda_hinge * L_hinge, with the reference's gating (a term whose weight is 0 is not evaluated).
+    lambda_dssim > 0 replaces Ll1 by (1 - lambda_dssim) * Ll1 + lambda_dssim * (1 - SSIM(blurred, gt)).
     depths [F,1,H,W] (query()['depths']), opacity = gaussians._opacity."""
-    loss = blur_photometric_loss(blurred, subframes, gt, lambda_t_smooth)
+    loss = photometric_loss(blurred, subframes, gt, lambda_t_smooth, lambda_dssim)
     if lambda_depth_tv > 0.0:
         loss = loss + lambda_depth_tv * tv_loss(depths)
     if lambda_hinge > 0.0:

@@ -5,6 +5,7 @@ Mirrors test.py of taekkii/deblurgs:
   OptimPoseModel        test.py:39-91    per-view unit quaternion (XYZW, `roma`'s convention) + w2c translation
   optimize_test_pose    test.py:131-186  iNeRF-style loop: L1(render, gt), Adam(rot 5e-5, trans 5e-4, eps 1e-15),
                                          StepLR(step = iters / 20, gamma 0.9), views visited in shuffled epochs
+  evaluate_views        test.py:401-439  per-view PSNR / SSIM of the renders against original_image (no LPIPS)
 `roma` is not a dependency here: the quaternion algebra lives in `pose.py`. Rendering goes through the
 drop-in `renderer.render` (single view) and the update through `params.FusedAdam`.
 """
@@ -16,6 +17,7 @@ import torch
 import torch.nn as nn
 
 from . import renderer
+from .loss import psnr, ssim
 from .params import FusedAdam
 from .pose import rotmat_to_unitquat, unitquat_to_rotmat
 
@@ -97,3 +99,21 @@ def optimize_test_pose(cams, gaussians, bg_color, num_iter_per_view=2000, tone_m
     with torch.no_grad():
         refined = [model(i) for i in range(n)]
     return refined, history
+
+
+def evaluate_views(cams, gaussians, bg_color, tone_mapping=None):
+    """Image quality of a scene at `cams` (e.g. the cameras optimize_test_pose returns): each view rendered without
+    gradients, tone-mapped if given, clamped to [0,1] and scored against cam.original_image with one batched SSIM call
+    and PSNR.  Returns {"psnr": [per view], "ssim": [per view], "psnr_mean": float, "ssim_mean": float}."""
+    with torch.no_grad():
+        renders = []
+        for cam in cams:
+            image = renderer.render(cam, gaussians, bg_color)["render"]
+            if tone_mapping is not None:
+                image = tone_mapping(image)
+            renders.append(image.clamp(0.0, 1.0))
+        pred = torch.stack(renders)
+        gt = torch.stack([cam.original_image[0:3] for cam in cams]).to(pred)
+        ssims = ssim(pred, gt, size_average=False).tolist()
+        psnrs = psnr(pred, gt)[:, 0].tolist()
+    return {"psnr": psnrs, "ssim": ssims, "psnr_mean": sum(psnrs) / len(psnrs), "ssim_mean": sum(ssims) / len(ssims)}

@@ -9,16 +9,19 @@ What the reference's train.py does per iteration (train.py:120-215), with this r
   gaussians.training_setup(opt)                     GaussianParams.training_setup(...)                (FusedAdam, 1 launch/step)
   camera_motion_module.add_training_setup(...)      same name
   query(cam_idx) -> F x render(), stack, mean       query(cam_idx): ONE batched forward for the F sub-frames
-  l1_loss + lambda * batchwise_smoothness_loss      blur_photometric_loss (one kernel each way)
+  l1_loss + lambda * batchwise_smoothness_loss      training_loss (fused L1 / smoothness kernel each way)
+  (1-l) * L1 + l * (1 - ssim)   (--lambda-dssim)    training_loss(..., lambda_dssim=l)  (fused SSIM kernel each way)
   loss.backward()                                   one batched backward (+ pose kernel backward)
   for pkg in render_pkgs: add_densification_stats   add_densification_stats_blurry(pkg)  (computed in the backward)
   clip_grad_value_; optimizer.step(); zero_grad     optimizer.step(clip_grad_value=...); zero_grad
   gaussians.densify_and_prune(threshold, extent)    same name (deblurgs_b200/densify.py; optimizer state follows)
 
 The "ground truth" blurry images are rendered from a hidden scene / trajectories; training starts from perturbed
-colours, opacities and trajectories and must bring the photometric loss down.
+colours, opacities and trajectories and must bring the photometric loss down.  At the end the deblurred scene is
+scored the way DeblurGS is judged: the trained and the hidden scene rendered sharp at each view's true mid-exposure
+pose, PSNR / SSIM before and after training (refine.evaluate_views).
 
-  python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000]
+  python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000] [--lambda-dssim 0.2]
 """
 import argparse
 import os
@@ -28,9 +31,10 @@ import time
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from deblurgs_b200 import blur_photometric_loss, synthetic  # noqa: E402
+from deblurgs_b200 import renderer, synthetic, training_loss  # noqa: E402
 from deblurgs_b200.motion import CameraMotionModule, GaussianParams  # noqa: E402
 from deblurgs_b200.pose import bezier_se3_poses  # noqa: E402
+from deblurgs_b200.refine import evaluate_views  # noqa: E402
 
 
 class RefCamera:
@@ -43,6 +47,16 @@ class RefCamera:
         self.original_image = None
 
 
+class SharpView:
+    """A camera at one fixed pose (what renderer.render reads), scored against `original_image`."""
+
+    def __init__(self, cam, view, proj, campos, image):
+        self.image_width, self.image_height = cam.width, cam.height
+        self.FoVx, self.FoVy = cam.fovx, cam.fovy
+        self.world_view_transform, self.full_proj_transform, self.camera_center = view, proj, campos
+        self.original_image = image
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=200)
@@ -52,6 +66,7 @@ def main():
     ap.add_argument("--width", type=int, default=200)
     ap.add_argument("--height", type=int, default=136)
     ap.add_argument("--densify-every", type=int, default=100, help="0: never")
+    ap.add_argument("--lambda-dssim", type=float, default=0.0, help="weight of the D-SSIM term (3DGS uses 0.2)")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
@@ -86,12 +101,17 @@ def main():
     opt = gauss.training_setup(position_lr_init=1.6e-5, feature_lr=0.01, opacity_lr=0.02, scaling_lr=0.002,
                                rotation_lr=0.001)
     # mid-trajectory camera pose of every view -> (c2w rotation, camera position), as COLMAP would give them
-    mid_R, mid_t = [], []
+    mid_R, mid_t, sharp = [], [], []
     for t in true_traj:
-        view, _, campos = bezier_se3_poses(t.ctrl_trans, t.ctrl_rot, torch.tensor([0.5], device=dev),
-                                           cams[0].projection_matrix)
+        view, proj, campos = bezier_se3_poses(t.ctrl_trans, t.ctrl_rot, torch.tensor([0.5], device=dev),
+                                              cams[0].projection_matrix)
         mid_R.append(view[0, :3, :3])
         mid_t.append(campos[0])
+        with torch.no_grad():     # the hidden scene, sharp at the true mid-exposure pose: what deblurring should recover
+            v = SharpView(cam, view[0], proj[0], campos[0], None)
+            v.original_image = renderer.render(v, truth, bg)["render"].clamp(0.0, 1.0)
+        sharp.append(v)
+    before = evaluate_views(sharp, gauss, bg)
     cmm = CameraMotionModule.from_poses(cams, torch.stack(mid_R), torch.stack(mid_t), curve_order=order,
                                         num_subframes=F)
     cmm.link_gaussian(gauss)
@@ -103,7 +123,8 @@ def main():
         idx = it % args.views
         lam = lam0 * (lam1 / lam0) ** (it / max(args.iters - 1, 1))
         out = cmm.query(idx, "all", background=bg)
-        loss = blur_photometric_loss(out["blurred"], out["subframes"], out["gt"], lam)
+        loss = training_loss(out["blurred"], out["subframes"], out["gt"], lambda_t_smooth=lam,
+                             lambda_dssim=args.lambda_dssim)
         loss.backward()
         with torch.no_grad():
             gauss.add_densification_stats_blurry(out["batched"])    # train.py:188-193, from the backward's epilogue
@@ -122,6 +143,9 @@ def main():
           "densification: %d Gaussians seen, max screen radius %d px"
           % (args.iters, dt, 1e3 * dt / args.iters, log[0][1], log[-1][1], int((gauss.denom > 0).sum()),
              int(gauss.max_radii2D.max())))
+    after = evaluate_views(sharp, gauss, bg)
+    print("sharp mid-exposure views vs the hidden scene: PSNR %.2f -> %.2f dB, SSIM %.4f -> %.4f"
+          % (before["psnr_mean"], after["psnr_mean"], before["ssim_mean"], after["ssim_mean"]))
     assert log[-1][1] < 0.8 * log[0][1], "training did not reduce the loss"
 
 

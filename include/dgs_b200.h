@@ -322,6 +322,23 @@ int dgs_hinge_l2_forward(int64_t n, const float* x, float* loss_out, double* scr
 int dgs_hinge_l2_backward(int64_t n, const float* x, const float* grad_out, float* dL_dx, void* stream);
 
 /*
+ * SSIM (3DGS utils/loss_utils.py `ssim`, window 11, sigma 1.5, zero padding, C1 = 0.01^2, C2 = 0.03^2) of two
+ * [N, C, H, W] fp32 stacks, N * C <= 65535.
+ *   forward:  ssim_out [1 + N] = (mean over all N*C*H*W map values, mean of image 0, ..., mean of image N-1);
+ *             scratch = dgs_ssim_scratch_bytes(N, C, H, W) bytes (one double per 32x16 tile of every plane; 0 for an
+ *             invalid size).  The partial sums are reduced in a fixed order: the result does not vary between calls.
+ *             maps [3, N, C, H, W] (or NULL when no gradient is wanted) receives dS/dmu1, dS/dsigma1^2, dS/dsigma12.
+ *   backward: dL_dimg1 [N, C, H, W] written from the forward's maps; img2 is a constant.  grad_out = device pointer
+ *             to dL/dssim (NULL = 1): one value (per_image == 0, the overall mean) or N values (per_image != 0).
+ * No allocation and no host synchronisation inside: both calls can be captured in a CUDA graph.
+ */
+size_t dgs_ssim_scratch_bytes(int N, int C, int H, int W);
+int dgs_ssim_forward(int N, int C, int H, int W, const float* img1, const float* img2, float* ssim_out,
+                     double* scratch, float* maps, void* stream);
+int dgs_ssim_backward(int N, int C, int H, int W, const float* img1, const float* img2, const float* maps,
+                      const float* grad_out, int per_image, float* dL_dimg1, void* stream);
+
+/*
  * Gaussian parameter store, the steps either side of the rasterizer (SURVEY.md 8f rank 3).
  *
  * dgs_activate_forward replaces the four getters `render` reads -- get_features (cat of _features_dc
