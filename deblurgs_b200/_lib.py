@@ -34,6 +34,9 @@ SIGNATURES = {
     "dgs_blur_forward_hint": (_i, [ALLOC_FN, _p, ALLOC_FN, _p, ALLOC_FN, _p,
                                    _i, _i, _i, _i] + _FWD_COMMON +
                               [_i, _i, _p, _p, _p, _p, _f, _i64, C.POINTER(_i64), _p]),
+    "dgs_blur_forward_aa": (_i, [ALLOC_FN, _p, ALLOC_FN, _p, ALLOC_FN, _p,
+                                 _i, _i, _i, _i] + _FWD_COMMON +
+                            [_i, _i, _p, _p, _p, _p, _f, _i64, C.POINTER(_i64), _i, _p]),
     "dgs_blur_forward_status": (_i, [_p, _i, _i, C.POINTER(_i64), C.POINTER(_i), _p]),
     "dgs_blur_forward_status_offset": (C.c_size_t, [_i, _i]),
     "dgs_blur_backward_scratch_bytes": (C.c_size_t, [_i, _i]),
@@ -41,6 +44,8 @@ SIGNATURES = {
                           [_i, _p, _p, _p, _p, _p, _p, _p, _f, _p] + [_p] * 11 + [_p]),
     "dgs_blur_backward_range": (_i, [_i, _i, _i, _i, _i64] + _FWD_COMMON +
                                 [_i, _p, _p, _p, _p, _p, _p, _p, _f, _p] + [_p] * 11 + [_i64, _i64, _i, _p]),
+    "dgs_blur_backward_range_aa": (_i, [_i, _i, _i, _i, _i64] + _FWD_COMMON +
+                                   [_i, _p, _p, _p, _p, _p, _p, _p, _f, _p] + [_p] * 11 + [_i64, _i64, _i, _i, _p]),
     "dgs_forward": (_i, [ALLOC_FN, _p, ALLOC_FN, _p, ALLOC_FN, _p,
                          _i, _i, _i] + _FWD_COMMON + [_i, _i, _p, _p, _p, C.POINTER(_i64), _p]),
     "dgs_backward": (_i, [_i, _i, _i, _i64] + _FWD_COMMON +

@@ -254,7 +254,7 @@ int dgs_key_bits(int width, int height, int F, int* tile_bits, int* subframe_bit
     return DGS_OK;
 }
 
-/* Shared implementation of dgs_blur_forward / dgs_blur_forward_hint.
+/* Shared implementation of dgs_blur_forward / dgs_blur_forward_hint / dgs_blur_forward_aa.
  *   capacity_hint == 0  exact mode: the host waits for D after the scan stage (one synchronisation, like the
  *                       reference's rasterizer_impl.cu:287) and sizes the binning buffer from it.
  *   capacity_hint  > 0  speculative mode: the binning buffer is sized from the hint and every kernel of the view is
@@ -276,9 +276,10 @@ static int blur_forward_impl(
     int prefiltered, int use_sigmoid,
     float* out_color, float* out_depth, int* radii,
     float* out_blur, float blur_denominator,
-    int64_t capacity_hint, int64_t* num_rendered, void* stream)
+    int64_t capacity_hint, int64_t* num_rendered, int antialiasing, void* stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
+    if (antialiasing != 0 && antialiasing != 1) return fail(DGS_ERR_INVALID_ARGUMENT, "antialiasing must be 0 or 1");
     FwdParams p;
     memset(&p, 0, sizeof(p));
     int rc = fill_params(p, P, F, sh_coeffs, background, width, height, means3D, shs, colors_precomp,
@@ -321,7 +322,7 @@ static int blur_forward_impl(
     const bool speculative = capacity_hint > 0;
     if (N > 0) {
         DGS_CUDA(cudaMemsetAsync(geom + G.status, 0, G.rect - G.status, st), "status memset");   // status .. ticket
-        { StageTimer t(ST_PREPROCESS_FWD, st, 1); launch_preprocess_fwd(p, sh_degree, st); }
+        { StageTimer t(ST_PREPROCESS_FWD, st, 1); launch_preprocess_fwd(p, sh_degree, antialiasing != 0, st); }
         {
             // stage 1: depth order of the Gaussians of every sub-frame (segmented sort on the 32 depth bits)
             StageTimer t(ST_DEPTH_SORT, st, 12);
@@ -437,7 +438,7 @@ int dgs_blur_forward(
                              sh_coeffs, background, width, height, means3D, shs, colors_precomp, opacities, scales,
                              scale_modifier, rotations, cov3D_precomp, viewmatrix, projmatrix, campos, tan_fovx,
                              tan_fovy, z_near, z_far, prefiltered, use_sigmoid, out_color, out_depth, radii, out_blur,
-                             blur_denominator, 0, num_rendered, stream);
+                             blur_denominator, 0, num_rendered, 0, stream);
 }
 
 int dgs_blur_forward_hint(
@@ -459,7 +460,29 @@ int dgs_blur_forward_hint(
                              sh_coeffs, background, width, height, means3D, shs, colors_precomp, opacities, scales,
                              scale_modifier, rotations, cov3D_precomp, viewmatrix, projmatrix, campos, tan_fovx,
                              tan_fovy, z_near, z_far, prefiltered, use_sigmoid, out_color, out_depth, radii, out_blur,
-                             blur_denominator, binning_capacity, num_rendered, stream);
+                             blur_denominator, binning_capacity, num_rendered, 0, stream);
+}
+
+int dgs_blur_forward_aa(
+    dgs_alloc_fn geom_alloc, void* geom_ctx, dgs_alloc_fn binning_alloc, void* binning_ctx,
+    dgs_alloc_fn image_alloc, void* image_ctx,
+    int P, int F, int sh_degree, int sh_coeffs,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far,
+    int prefiltered, int use_sigmoid,
+    float* out_color, float* out_depth, int* radii,
+    float* out_blur, float blur_denominator,
+    int64_t binning_capacity, int64_t* num_rendered, int antialiasing, void* stream)
+{
+    return blur_forward_impl(geom_alloc, geom_ctx, binning_alloc, binning_ctx, image_alloc, image_ctx, P, F, sh_degree,
+                             sh_coeffs, background, width, height, means3D, shs, colors_precomp, opacities, scales,
+                             scale_modifier, rotations, cov3D_precomp, viewmatrix, projmatrix, campos, tan_fovx,
+                             tan_fovy, z_near, z_far, prefiltered, use_sigmoid, out_color, out_depth, radii, out_blur,
+                             blur_denominator, binning_capacity, num_rendered, antialiasing, stream);
 }
 
 size_t dgs_blur_forward_status_offset(int P, int F)
@@ -489,7 +512,8 @@ size_t dgs_blur_backward_scratch_bytes(int P, int F)
     return align_up(N * 12 * sizeof(float)) + align_up((size_t)F * 32 * sizeof(double)) + 256;
 }
 
-int dgs_blur_backward_range(
+// Shared implementation of dgs_blur_backward_range / dgs_blur_backward_range_aa.
+static int blur_backward_impl(
     int P, int F, int sh_degree, int sh_coeffs, int64_t num_rendered,
     const float* background, int width, int height,
     const float* means3D, const float* shs, const float* colors_precomp,
@@ -504,9 +528,10 @@ int dgs_blur_backward_range(
     float* dL_dmeans2D, float* dL_dmeans3D, float* dL_dsh, float* dL_dopacity,
     float* dL_dscales, float* dL_drotations, float* dL_dcolors_precomp, float* dL_dcov3D_precomp,
     float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
-    int64_t g_begin, int64_t g_end, int stages, void* stream)
+    int64_t g_begin, int64_t g_end, int stages, int antialiasing, void* stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
+    if (antialiasing != 0 && antialiasing != 1) return fail(DGS_ERR_INVALID_ARGUMENT, "antialiasing must be 0 or 1");
     if (g_begin < 0 || g_end > P || g_begin > g_end) return fail(DGS_ERR_INVALID_ARGUMENT, "bad Gaussian range");
     BwdParams b;
     memset(&b, 0, sizeof(b));
@@ -572,11 +597,63 @@ int dgs_blur_backward_range(
     }
     if ((stages & DGS_BWD_GAUSSIANS) && g_end > g_begin) {
         StageTimer t(ST_PREPROCESS_BWD, st, colors_precomp ? 1 : 2);
-        launch_preprocess_bwd(b, sh_degree, st);
+        launch_preprocess_bwd(b, sh_degree, antialiasing != 0, st);
     }
     if (stages & DGS_BWD_FINISH) { StageTimer t(ST_PREPROCESS_BWD, st, 1); launch_pose_finalize(b, st); }
     DGS_CUDA(cudaGetLastError(), "backward launch");
     return DGS_OK;
+}
+
+int dgs_blur_backward_range(
+    int P, int F, int sh_degree, int sh_coeffs, int64_t num_rendered,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far, int use_sigmoid,
+    const int* radii,
+    const char* geom_buffer, const char* binning_buffer, const char* image_buffer,
+    const float* dL_dpix, const float* dL_dpixdepth, const float* dL_dblur, float blur_denominator,
+    char* scratch,
+    float* dL_dmeans2D, float* dL_dmeans3D, float* dL_dsh, float* dL_dopacity,
+    float* dL_dscales, float* dL_drotations, float* dL_dcolors_precomp, float* dL_dcov3D_precomp,
+    float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
+    int64_t g_begin, int64_t g_end, int stages, void* stream)
+{
+    return blur_backward_impl(P, F, sh_degree, sh_coeffs, num_rendered, background, width, height, means3D, shs,
+                              colors_precomp, opacities, scales, scale_modifier, rotations, cov3D_precomp, viewmatrix,
+                              projmatrix, campos, tan_fovx, tan_fovy, z_near, z_far, use_sigmoid, radii, geom_buffer,
+                              binning_buffer, image_buffer, dL_dpix, dL_dpixdepth, dL_dblur, blur_denominator, scratch,
+                              dL_dmeans2D, dL_dmeans3D, dL_dsh, dL_dopacity, dL_dscales, dL_drotations,
+                              dL_dcolors_precomp, dL_dcov3D_precomp, dL_dviewmatrix, dL_dprojmatrix, densify_stats,
+                              g_begin, g_end, stages, 0, stream);
+}
+
+int dgs_blur_backward_range_aa(
+    int P, int F, int sh_degree, int sh_coeffs, int64_t num_rendered,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far, int use_sigmoid,
+    const int* radii,
+    const char* geom_buffer, const char* binning_buffer, const char* image_buffer,
+    const float* dL_dpix, const float* dL_dpixdepth, const float* dL_dblur, float blur_denominator,
+    char* scratch,
+    float* dL_dmeans2D, float* dL_dmeans3D, float* dL_dsh, float* dL_dopacity,
+    float* dL_dscales, float* dL_drotations, float* dL_dcolors_precomp, float* dL_dcov3D_precomp,
+    float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
+    int64_t g_begin, int64_t g_end, int stages, int antialiasing, void* stream)
+{
+    return blur_backward_impl(P, F, sh_degree, sh_coeffs, num_rendered, background, width, height, means3D, shs,
+                              colors_precomp, opacities, scales, scale_modifier, rotations, cov3D_precomp, viewmatrix,
+                              projmatrix, campos, tan_fovx, tan_fovy, z_near, z_far, use_sigmoid, radii, geom_buffer,
+                              binning_buffer, image_buffer, dL_dpix, dL_dpixdepth, dL_dblur, blur_denominator, scratch,
+                              dL_dmeans2D, dL_dmeans3D, dL_dsh, dL_dopacity, dL_dscales, dL_drotations,
+                              dL_dcolors_precomp, dL_dcov3D_precomp, dL_dviewmatrix, dL_dprojmatrix, densify_stats,
+                              g_begin, g_end, stages, antialiasing, stream);
 }
 
 int dgs_blur_backward(

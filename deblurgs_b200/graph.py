@@ -27,7 +27,9 @@ class BlurryViewGraph:
         loss = step.replay()                   # 0-dim device tensor (static storage); .grad of every parameter is set
         ...optimizer.step()                    # .grad tensors are static storage owned by the graph (re-attached on replay)
         step.check()                           # after a synchronisation: re-captures + replays if the capacity was exceeded
-    `parameters` (default: the Gaussians' and the trajectory's) get their .grad from the captured backward."""
+    `parameters` (default: the Gaussians' and the trajectory's) get their .grad from the captured backward.
+    The store's `antialiasing` flag is read when the step is captured and is part of the graph: a replay after the flag
+    was changed raises DgsError (build a new BlurryViewGraph for the other setting) instead of rendering the old one."""
 
     def __init__(self, cmm, cam_idx, background, gt_shape, lambda_t_smooth=0.0, parameters=None, pre_backward=None,
                  caller_owned_grads=(), capacity_margin=1.25, post_backward=None, render_fn=None,
@@ -51,6 +53,7 @@ class BlurryViewGraph:
         self.status_host = torch.zeros(6, dtype=torch.int32).pin_memory()
         self.graph, self.loss, self.out, self.capacity = None, None, None, 0
         self.recaptures = 0
+        self.antialiasing = self._store_antialiasing()
         self._capture(None)
 
     # ------------------------------------------------------------------------------------------
@@ -67,6 +70,9 @@ class BlurryViewGraph:
         if self.post_backward is not None:
             self.post_backward()
         return out, loss.detach()
+
+    def _store_antialiasing(self):
+        return bool(getattr(self.cmm.gaussians, "antialiasing", False))
 
     def _reset_grads(self):
         for p in self.params:
@@ -113,6 +119,9 @@ class BlurryViewGraph:
 
     # ------------------------------------------------------------------------------------------
     def replay(self):
+        if self._store_antialiasing() != self.antialiasing:
+            raise _lib.DgsError("the store's antialiasing flag changed since this step was captured (captured with "
+                                "antialiasing=%s): build a new BlurryViewGraph for the new setting" % self.antialiasing)
         self.graph.replay()
         for p, g in zip(self.params, self.grads):      # re-attach if someone replaced or cleared a .grad meanwhile
             if p.grad is not g:

@@ -83,7 +83,8 @@ class GaussianParams(DensificationMixin):
     (`densify.DensificationMixin`)."""
 
     def __init__(self, xyz, features_dc, features_rest, scaling, rotation, opacity, active_sh_degree,
-                 z_near=0.2, z_far=100.0, use_sigmoid=False, scale_lower_bound=0.0, use_isotropic=False):
+                 z_near=0.2, z_far=100.0, use_sigmoid=False, scale_lower_bound=0.0, use_isotropic=False,
+                 antialiasing=False):
         self._xyz = nn.Parameter(xyz.contiguous())
         self._features_dc = nn.Parameter(features_dc.contiguous())
         self._features_rest = nn.Parameter(features_rest.contiguous())
@@ -96,6 +97,7 @@ class GaussianParams(DensificationMixin):
         self.use_sigmoid = use_sigmoid
         self.scale_lower_bound = scale_lower_bound
         self.use_isotropic = use_isotropic
+        self.antialiasing = antialiasing   # screen-space antialiasing filter, read by renderer.render / render_blurry
         self.optimizer = None
         self.grad_sink = None      # optional dist.FlatGradBuffer.for_gaussians(self): gradients all-reduced under the backward
 

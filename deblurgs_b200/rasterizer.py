@@ -81,8 +81,9 @@ _ASYNC = None   # None, or {"capacity": int, "geoms": [(tensor, P, F), ...]}
 
 def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                      viewmatrix, projmatrix, campos, bg, H, W, tanfovx, tanfovy, scale_modifier,
-                     z_near, z_far, sh_degree, prefiltered, use_sigmoid, want_blur, blur_denominator, exact=False):
-    """Runs dgs_blur_forward_hint. viewmatrix/projmatrix [F,4,4], campos [F,3]."""
+                     z_near, z_far, sh_degree, prefiltered, use_sigmoid, want_blur, blur_denominator, exact=False,
+                     antialiasing=False):
+    """Runs dgs_blur_forward_aa. viewmatrix/projmatrix [F,4,4], campos [F,3]."""
     lib = _lib.load()
     _require_cuda(means3D, "means3D")
     if means3D.dim() != 2 or means3D.shape[1] != 3:
@@ -109,7 +110,7 @@ def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, 
     if _ASYNC is not None:
         hint = int(_ASYNC["capacity"])
     with torch.cuda.device(dev):
-        rc = lib.dgs_blur_forward_hint(
+        rc = lib.dgs_blur_forward_aa(
             geom.cb, None, binning.cb, None, img.cb, None,
             P, F, int(sh_degree), int(M),
             _lib.ptr(bg), int(W), int(H),
@@ -121,12 +122,13 @@ def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, 
             int(bool(prefiltered)), int(bool(use_sigmoid)),
             _lib.ptr(color), _lib.ptr(depth), _lib.ptr(radii),
             _lib.ptr(blur), float(blur_denominator),
-            int(hint), None if _ASYNC is not None else C.byref(num_rendered), _stream_ptr(dev))
+            int(hint), None if _ASYNC is not None else C.byref(num_rendered), int(bool(antialiasing)),
+            _stream_ptr(dev))
     # drop the ctypes callbacks: they close over the _Buffer objects (a reference cycle), and a cycle
     # would keep hundreds of MB of state buffers alive until Python's cyclic GC runs, forcing the caching
     # allocator to cudaMalloc fresh blocks every step in the meantime
     geom.cb = binning.cb = img.cb = None
-    _lib.check(rc, "dgs_blur_forward_hint")
+    _lib.check(rc, "dgs_blur_forward_aa")
     if _ASYNC is not None:
         _ASYNC["geoms"].append((geom.t, P, F))
         return color, depth, radii, blur, -1, geom.t, binning.t, img.t    # -1: number of duplicates unknown on the host
@@ -142,8 +144,8 @@ def _backward_batched(P, F, M, num_rendered, means3D, sh, colors_precomp, opacit
                       cov3Ds_precomp, viewmatrix, projmatrix, campos, bg, H, W, tanfovx, tanfovy,
                       scale_modifier, z_near, z_far, sh_degree, use_sigmoid, radii, geom, binning, img,
                       grad_color, grad_depth, want_means2D, grad_blur=None, blur_denominator=1.0, want_stats=False,
-                      ranges=None, outputs=None, on_range=None):
-    """Runs dgs_blur_backward_range.  ranges: list of (g0, g1) covering [0, P) -- the per-Gaussian stage is launched
+                      ranges=None, outputs=None, on_range=None, antialiasing=False):
+    """Runs dgs_blur_backward_range_aa (`antialiasing` must be the forward's).  ranges: list of (g0, g1) covering [0, P) -- the per-Gaussian stage is launched
     once per range and `on_range(g0, g1, out)` is called after each (e.g. to start a collective on those rows while
     the next range computes); outputs: preallocated (dmeans3D, dsh, dopacity, dscales, drot) to write into."""
     lib = _lib.load()
@@ -176,7 +178,7 @@ def _backward_batched(P, F, M, num_rendered, means3D, sh, colors_precomp, opacit
 
     def call(g0, g1, stages):
         with torch.cuda.device(dev):
-            rc = lib.dgs_blur_backward_range(
+            rc = lib.dgs_blur_backward_range_aa(
                 P, F, int(sh_degree), int(M), int(num_rendered),
                 _lib.ptr(bg), int(W), int(H),
                 _lib.ptr(means3D), _lib.ptr(sh), _lib.ptr(colors_precomp),
@@ -189,8 +191,9 @@ def _backward_batched(P, F, M, num_rendered, means3D, sh, colors_precomp, opacit
                 _lib.ptr(scratch),
                 _lib.ptr(dmeans2D), _lib.ptr(dmeans3D), _lib.ptr(dsh), _lib.ptr(dopacity),
                 _lib.ptr(dscales), _lib.ptr(drot), _lib.ptr(dcolors), _lib.ptr(dcov),
-                _lib.ptr(dview), _lib.ptr(dproj), _lib.ptr(stats), int(g0), int(g1), int(stages), _stream_ptr(dev))
-        _lib.check(rc, "dgs_blur_backward_range")
+                _lib.ptr(dview), _lib.ptr(dproj), _lib.ptr(stats), int(g0), int(g1), int(stages),
+                int(bool(antialiasing)), _stream_ptr(dev))
+        _lib.check(rc, "dgs_blur_backward_range_aa")
 
     if ranges is None:
         call(0, P, BWD_ALL)
@@ -213,11 +216,11 @@ def _empty_like_input(t):
 
 class _RasterizeGaussians(torch.autograd.Function):
     """Single view. Same argument order, saved state and gradient tuple as the reference's
-    `_RasterizeGaussians` (diff_gaussian_rasterization/__init__.py:48-170)."""
+    `_RasterizeGaussians` (diff_gaussian_rasterization/__init__.py:48-170), plus a trailing `antialiasing` flag."""
 
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                cov3Ds_precomp, viewmatrix, projmatrix, raster_settings):
+                cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, antialiasing=False):
         rs = raster_settings
         ctx.set_materialize_grads(False)   # an unused output (depth) arrives as None, not as a zero-filled image
         means3D_c, sh_c, colors_c = _f32c(means3D), _f32c(sh), _f32c(colors_precomp)
@@ -229,9 +232,10 @@ class _RasterizeGaussians(torch.autograd.Function):
         color, depth, radii, _, num_rendered, geom, binning, img = _forward_batched(
             means3D_c, sh_c, colors_c, opac_c, scales_c, rot_c, cov_c, view_c, proj_c, campos_c, bg_c,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near,
-            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, False, 1.0)
+            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, False, 1.0, antialiasing=antialiasing)
         ctx.raster_settings = rs
         ctx.num_rendered = num_rendered
+        ctx.antialiasing = bool(antialiasing)
         ctx.save_for_backward(colors_c, means3D_c, scales_c, rot_c, cov_c, radii, sh_c, opac_c, geom, binning,
                               img, view_c, proj_c, campos_c, bg_c)
         ctx.mark_non_differentiable(radii)
@@ -249,17 +253,18 @@ class _RasterizeGaussians(torch.autograd.Function):
         (dmeans2D, dmeans3D, dsh, dopacity, dscales, drot, dcolors, dcov, dview, dproj, _) = _backward_batched(
             P, 1, M, ctx.num_rendered, means3D, sh, colors_c, opac, scales, rot, cov, view, proj, campos, bg,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near, rs.z_far,
-            rs.sh_degree, rs.use_sigmoid, radii, geom, binning, img, gc, gd, True)
+            rs.sh_degree, rs.use_sigmoid, radii, geom, binning, img, gc, gd, True, antialiasing=ctx.antialiasing)
         # reference order: means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
         # cov3Ds_precomp, viewmatrix, projmatrix, raster_settings
         return (dmeans3D, dmeans2D[0], dsh if sh.numel() != 0 else None, dcolors, dopacity, dscales, drot, dcov,
-                dview[0], dproj[0], None)
+                dview[0], dproj[0], None, None)
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                        viewmatrix, projmatrix, raster_settings):
+                        viewmatrix, projmatrix, raster_settings, antialiasing=False):
+    """`antialiasing`: Mip-Splatting's screen-space filter (include/dgs_b200.h, dgs_blur_forward_aa)."""
     return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                     cov3Ds_precomp, viewmatrix, projmatrix, raster_settings)
+                                     cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, bool(antialiasing))
 
 
 class _RasterizeBlurry(torch.autograd.Function):
@@ -270,7 +275,8 @@ class _RasterizeBlurry(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder=None):
+                viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder=None,
+                antialiasing=False):
         rs = raster_settings
         # outputs the loss does not use (typically the [F,3,H,W] / [F,1,H,W] stacks when only `blurred` is) arrive
         # as None in backward instead of zero-filled tensors the kernel would then have to read
@@ -284,10 +290,11 @@ class _RasterizeBlurry(torch.autograd.Function):
         color, depth, radii, blur, num_rendered, geom, binning, img = _forward_batched(
             means3D_c, sh_c, colors_c, opac_c, scales_c, rot_c, cov_c, view_c, proj_c, campos_c, bg_c,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near,
-            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, True, denom)
+            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing)
         ctx.raster_settings = rs
         ctx.num_rendered = num_rendered
         ctx.denom = denom
+        ctx.antialiasing = bool(antialiasing)
         ctx.want_means2D = means2D is not None and means2D.requires_grad
         ctx.save_for_backward(colors_c, means3D_c, scales_c, rot_c, cov_c, radii, sh_c, opac_c, geom, binning,
                               img, view_c, proj_c, campos_c, bg_c)
@@ -311,13 +318,13 @@ class _RasterizeBlurry(torch.autograd.Function):
             P, F, M, ctx.num_rendered, means3D, sh, colors_c, opac, scales, rot, cov, view, proj, campos, bg,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near, rs.z_far,
             rs.sh_degree, rs.use_sigmoid, radii, geom, binning, img, gc, gd, ctx.want_means2D, gb, ctx.denom,
-            holder is not None)
+            holder is not None, antialiasing=ctx.antialiasing)
         if holder is not None:
             # denominator of the view's blur = number of sub-frames of the WHOLE view (a rank that renders a shard of
             # the sub-frames still normalises its visible-count by all of them, train.py:193: 1 / len(render_pkgs))
             holder.fill(stats, ctx.denom)
         return (dmeans3D, dmeans2D, dsh if sh.numel() != 0 else None, dcolors, dopacity, dscales, drot, dcov,
-                dview, dproj, None, None, None, None)
+                dview, dproj, None, None, None, None, None)
 
 
 class _RenderStoreBlurry(torch.autograd.Function):
@@ -330,7 +337,8 @@ class _RenderStoreBlurry(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, xyz, f_dc, f_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix, campos,
-                raster_settings, blur_denominator, stats_holder, scale_lb, isotropic, grad_sink, n_ranges):
+                raster_settings, blur_denominator, stats_holder, scale_lb, isotropic, grad_sink, n_ranges,
+                antialiasing=False):
         lib = _lib.load()
         rs = raster_settings
         _require_cuda(xyz, "xyz")
@@ -355,8 +363,9 @@ class _RenderStoreBlurry(torch.autograd.Function):
         color, depth, radii, blur, num_rendered, geom, binning, img = _forward_batched(
             xyz_c, shs, None, opac, scales, rots, None, view_c, proj_c, campos_c, bg_c, rs.image_height,
             rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near, rs.z_far, rs.sh_degree,
-            rs.prefiltered, rs.use_sigmoid, True, denom)
+            rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing)
         ctx.raster_settings, ctx.num_rendered, ctx.denom = rs, num_rendered, denom
+        ctx.antialiasing = bool(antialiasing)
         ctx.want_means2D = means2D is not None and means2D.requires_grad
         ctx.stats_holder, ctx.sink, ctx.n_ranges = stats_holder, grad_sink, max(1, int(n_ranges))
         ctx.meta = (M, bool(isotropic), f_dc.shape, f_rest.shape)
@@ -409,21 +418,22 @@ class _RenderStoreBlurry(torch.autograd.Function):
             P, F, M, ctx.num_rendered, xyz, shs, None, opac, scales, rots, None, view, proj, campos, bg,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near, rs.z_far,
             rs.sh_degree, rs.use_sigmoid, radii, geom, binning, img, gc, gd, ctx.want_means2D, gb, ctx.denom,
-            holder is not None, ranges=ranges, outputs=(dxyz, dsh, dopac, dscales, drots), on_range=after_range)
+            holder is not None, ranges=ranges, outputs=(dxyz, dsh, dopac, dscales, drots), on_range=after_range,
+            antialiasing=ctx.antialiasing)
         if holder is not None:
             holder.fill(stats, ctx.denom)
         if sink is not None:
             sink.finish()
-            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 8
-        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 8
+            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 9
+        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 9
 
 
 def render_store_blurry(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix,
                         campos, raster_settings, blur_denominator=None, stats_holder=None, scale_lower_bound=0.0,
-                        isotropic=False, grad_sink=None, n_ranges=4):
+                        isotropic=False, grad_sink=None, n_ranges=4, antialiasing=False):
     return _RenderStoreBlurry.apply(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix,
                                     projmatrix, campos, raster_settings, blur_denominator, stats_holder,
-                                    scale_lower_bound, isotropic, grad_sink, n_ranges)
+                                    scale_lower_bound, isotropic, grad_sink, n_ranges, bool(antialiasing))
 
 
 class DensificationStats:
@@ -450,20 +460,25 @@ class DensificationStats:
 
 
 def rasterize_blurry(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                     viewmatrix, projmatrix, campos, raster_settings, blur_denominator=None, stats_holder=None):
+                     viewmatrix, projmatrix, campos, raster_settings, blur_denominator=None, stats_holder=None,
+                     antialiasing=False):
     empty = torch.Tensor([])
     return _RasterizeBlurry.apply(
         means3D, means2D, sh if sh is not None else empty,
         colors_precomp if colors_precomp is not None else empty, opacities,
         scales if scales is not None else empty, rotations if rotations is not None else empty,
         cov3Ds_precomp if cov3Ds_precomp is not None else empty,
-        viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder)
+        viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder, bool(antialiasing))
 
 
 class GaussianRasterizer(nn.Module):
-    def __init__(self, raster_settings):
+    """`antialiasing` is a constructor argument, not a settings field: GaussianRasterizationSettings keeps the
+    reference's 13 fields."""
+
+    def __init__(self, raster_settings, antialiasing=False):
         super().__init__()
         self.raster_settings = raster_settings
+        self.antialiasing = bool(antialiasing)
 
     def markVisible(self, positions, viewmatrix=None, projmatrix=None):
         """Frustum test. The reference reads `raster_settings.viewmatrix`, a field that no longer
@@ -507,4 +522,4 @@ class GaussianRasterizer(nn.Module):
             cov3D_precomp = torch.Tensor([])
 
         return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
-                                   cov3D_precomp, viewmatrix, projmatrix, raster_settings)
+                                   cov3D_precomp, viewmatrix, projmatrix, raster_settings, self.antialiasing)

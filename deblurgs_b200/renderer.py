@@ -17,6 +17,7 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
 
     Also tolerates the upstream-3DGS call form render(cam, pc, pipe, bg_color, ...): a third
     positional argument that is not a Tensor is taken to be `pipe` and ignored.
+    Antialiasing follows `pc.antialiasing` (off when the store has no such attribute).
     """
     if not torch.is_tensor(bg_color):
         bg_color = scaling_modifier
@@ -47,7 +48,7 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
         prefiltered=False,
         debug=False,
     )
-    rasterizer = GaussianRasterizer(raster_settings=raster_settings)
+    rasterizer = GaussianRasterizer(raster_settings=raster_settings, antialiasing=getattr(pc, "antialiasing", False))
 
     shs = None
     colors_precomp = None
@@ -83,6 +84,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
     the sub-frames (e.g. from `pose.bezier_se3_poses`); `ref_cam` supplies image size and FoV.
     The Gaussian activations (pc.get_*) are evaluated once for the whole view, not once per sub-frame.
     Returns the reference's per-render dict with a leading sub-frame axis, plus "blurred".
+    Antialiasing follows `pc.antialiasing`, as in `render`.
     """
     xyz = pc.get_xyz
     F = world_view_transforms.shape[0]
@@ -115,7 +117,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
             pc._xyz, pc._features_dc, pc._features_rest, pc._scaling, pc._rotation, pc._opacity, screenspace_points,
             world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats,
             getattr(pc, "scale_lower_bound", 0.0), getattr(pc, "use_isotropic", False), sink,
-            int(getattr(sink, "n_ranges", 4)))
+            int(getattr(sink, "n_ranges", 4)), getattr(pc, "antialiasing", False))
         return {"render": color, "depth": depth, "blurred": blurred, "viewspace_points": screenspace_points,
                 "visibility_filter": radii > 0, "radii": radii, "densification": stats}
     if hasattr(pc, "get_activated"):
@@ -128,7 +130,8 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
         shs = None
     color, depth, radii, blurred = rasterize_blurry(
         xyz, screenspace_points, shs, override_color, opacities, scales, rotations, None,
-        world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats)
+        world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats,
+        getattr(pc, "antialiasing", False))
     return {"render": color,
             "depth": depth,
             "blurred": blurred,

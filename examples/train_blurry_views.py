@@ -19,14 +19,18 @@ What the reference's train.py does per iteration (train.py:120-215), with this r
 The "ground truth" blurry images are rendered from a hidden scene / trajectories; training starts from perturbed
 colours, opacities and trajectories and must bring the photometric loss down.  At the end the deblurred scene is
 scored the way DeblurGS is judged: the trained and the hidden scene rendered sharp at each view's true mid-exposure
-pose, PSNR / SSIM before and after training (refine.evaluate_views).
+pose, PSNR / SSIM before and after training (refine.evaluate_views), at full size and at half resolution (a camera of
+W/2 x H/2 with the same field of view, scored against the full-size sharp truth averaged over 2x2 pixel boxes).
+--antialiasing renders both the hidden and the trained scene with the screen-space antialiasing filter.
 
   python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000] [--lambda-dssim 0.2]
+                                        [--antialiasing]
 """
 import argparse
 import os
 import sys
 import time
+import types
 
 import torch
 
@@ -67,7 +71,10 @@ def main():
     ap.add_argument("--height", type=int, default=136)
     ap.add_argument("--densify-every", type=int, default=100, help="0: never")
     ap.add_argument("--lambda-dssim", type=float, default=0.0, help="weight of the D-SSIM term (3DGS uses 0.2)")
+    ap.add_argument("--antialiasing", action="store_true", help="screen-space antialiasing filter (Mip-Splatting)")
     args = ap.parse_args()
+    if args.width % 2 or args.height % 2:
+        raise SystemExit("--width and --height must be even (the half-resolution views average 2x2 pixel boxes)")
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
     order, F = 3, args.subframes
@@ -77,7 +84,7 @@ def main():
     bg = torch.zeros(3, device=dev)
 
     # ---- hidden truth: one trajectory per view around the base pose; blurry observations rendered from it
-    truth = GaussianParams.from_scene(scene)
+    truth = GaussianParams.from_scene(scene, antialiasing=args.antialiasing)
     cams = [RefCamera(cam, dev) for _ in range(args.views)]
     true_traj = [synthetic.make_trajectory(F, order, seed=10 + i).to(dev) for i in range(args.views)]
     base = torch.tensor([synthetic.BASE_SE3], dtype=torch.float32, device=dev).repeat(args.views, 1)
@@ -93,7 +100,7 @@ def main():
 
     # ---- the model being trained: same geometry, perturbed appearance; trajectories initialised from the mid pose
     g = torch.Generator().manual_seed(123)
-    gauss = GaussianParams.from_scene(scene)
+    gauss = GaussianParams.from_scene(scene, antialiasing=args.antialiasing)
     with torch.no_grad():
         gauss._features_dc.add_(0.5 * torch.randn(gauss._features_dc.shape, generator=g).to(dev))
         gauss._features_rest.mul_(0.0)
@@ -101,7 +108,8 @@ def main():
     opt = gauss.training_setup(position_lr_init=1.6e-5, feature_lr=0.01, opacity_lr=0.02, scaling_lr=0.002,
                                rotation_lr=0.001)
     # mid-trajectory camera pose of every view -> (c2w rotation, camera position), as COLMAP would give them
-    mid_R, mid_t, sharp = [], [], []
+    half_cam = types.SimpleNamespace(width=cam.width // 2, height=cam.height // 2, fovx=cam.fovx, fovy=cam.fovy)
+    mid_R, mid_t, sharp, sharp_half = [], [], [], []
     for t in true_traj:
         view, proj, campos = bezier_se3_poses(t.ctrl_trans, t.ctrl_rot, torch.tensor([0.5], device=dev),
                                               cams[0].projection_matrix)
@@ -111,7 +119,10 @@ def main():
             v = SharpView(cam, view[0], proj[0], campos[0], None)
             v.original_image = renderer.render(v, truth, bg)["render"].clamp(0.0, 1.0)
         sharp.append(v)
-    before = evaluate_views(sharp, gauss, bg)
+        # the same pose and field of view at half the resolution, scored against the truth box-filtered to that size
+        box = torch.nn.functional.avg_pool2d(v.original_image[None], 2)[0]
+        sharp_half.append(SharpView(half_cam, view[0], proj[0], campos[0], box))
+    before, before_half = evaluate_views(sharp, gauss, bg), evaluate_views(sharp_half, gauss, bg)
     cmm = CameraMotionModule.from_poses(cams, torch.stack(mid_R), torch.stack(mid_t), curve_order=order,
                                         num_subframes=F)
     cmm.link_gaussian(gauss)
@@ -143,9 +154,12 @@ def main():
           "densification: %d Gaussians seen, max screen radius %d px"
           % (args.iters, dt, 1e3 * dt / args.iters, log[0][1], log[-1][1], int((gauss.denom > 0).sum()),
              int(gauss.max_radii2D.max())))
-    after = evaluate_views(sharp, gauss, bg)
-    print("sharp mid-exposure views vs the hidden scene: PSNR %.2f -> %.2f dB, SSIM %.4f -> %.4f"
-          % (before["psnr_mean"], after["psnr_mean"], before["ssim_mean"], after["ssim_mean"]))
+    after, after_half = evaluate_views(sharp, gauss, bg), evaluate_views(sharp_half, gauss, bg)
+    for label, b, a in (("full size %dx%d" % (cam.width, cam.height), before, after),
+                        ("half size %dx%d" % (half_cam.width, half_cam.height), before_half, after_half)):
+        print("sharp mid-exposure views vs the hidden scene, %s, antialiasing %s: PSNR %.2f -> %.2f dB, SSIM %.4f -> %.4f"
+              % (label, "on" if args.antialiasing else "off", b["psnr_mean"], a["psnr_mean"], b["ssim_mean"],
+                 a["ssim_mean"]))
     assert log[-1][1] < 0.8 * log[0][1], "training did not reduce the loss"
 
 

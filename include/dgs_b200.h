@@ -186,6 +186,48 @@ int dgs_blur_backward_range(
     float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
     int64_t g_begin, int64_t g_end, int stages, void* stream);
 
+/*
+ * Antialiased rendering (Mip-Splatting's screen-space filter, DESIGN.md section 3).  Every projected 2-D covariance
+ * is dilated by 0.3 px^2 on its diagonal; with antialiasing = 1 the opacity a Gaussian blends with is scaled by
+ * rho = sqrt(max(det0 / det, 2.5e-5)) (det0, det: determinants before and after the dilation), so that a Gaussian
+ * narrower than a pixel keeps its integrated weight instead of rendering wider and more opaque.  Radii, tile
+ * rectangles, depth keys, sorted lists and conics are the same as with antialiasing = 0.
+ * Arguments are those of dgs_blur_forward_hint / dgs_blur_backward_range plus `antialiasing` (0 or 1; any other
+ * value fails with DGS_ERR_INVALID_ARGUMENT before any device work).  With 0 they are those two entry points.
+ * A backward must be called with the antialiasing value of the forward that filled its state buffers.
+ */
+int dgs_blur_forward_aa(
+    dgs_alloc_fn geom_alloc, void* geom_ctx,
+    dgs_alloc_fn binning_alloc, void* binning_ctx,
+    dgs_alloc_fn image_alloc, void* image_ctx,
+    int P, int F, int sh_degree, int sh_coeffs,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far,
+    int prefiltered, int use_sigmoid,
+    float* out_color, float* out_depth, int* radii,
+    float* out_blur, float blur_denominator,
+    int64_t binning_capacity, int64_t* num_rendered, int antialiasing, void* stream);
+int dgs_blur_backward_range_aa(
+    int P, int F, int sh_degree, int sh_coeffs, int64_t num_rendered,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far, int use_sigmoid,
+    const int* radii,
+    const char* geom_buffer, const char* binning_buffer, const char* image_buffer,
+    const float* dL_dpix, const float* dL_dpixdepth, const float* dL_dblur, float blur_denominator,
+    char* scratch,
+    float* dL_dmeans2D, float* dL_dmeans3D, float* dL_dsh, float* dL_dopacity,
+    float* dL_dscales, float* dL_drotations, float* dL_dcolors_precomp, float* dL_dcov3D_precomp,
+    float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
+    int64_t g_begin, int64_t g_end, int stages, int antialiasing, void* stream);
+
 /* Single-view pair: the reference's rasterize_gaussians / rasterize_gaussians_backward
  * (same argument meaning; F = 1 instance of the batched pair). */
 int dgs_forward(
