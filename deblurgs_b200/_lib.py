@@ -37,6 +37,9 @@ SIGNATURES = {
     "dgs_blur_forward_aa": (_i, [ALLOC_FN, _p, ALLOC_FN, _p, ALLOC_FN, _p,
                                  _i, _i, _i, _i] + _FWD_COMMON +
                             [_i, _i, _p, _p, _p, _p, _f, _i64, C.POINTER(_i64), _i, _p]),
+    "dgs_blur_forward_contrib": (_i, [ALLOC_FN, _p, ALLOC_FN, _p, ALLOC_FN, _p,
+                                      _i, _i, _i, _i] + _FWD_COMMON +
+                                 [_i, _i, _p, _p, _p, _p, _f, _i64, C.POINTER(_i64), _i, _p, _p, _p]),
     "dgs_blur_forward_status": (_i, [_p, _i, _i, C.POINTER(_i64), C.POINTER(_i), _p]),
     "dgs_blur_forward_status_offset": (C.c_size_t, [_i, _i]),
     "dgs_blur_backward_scratch_bytes": (C.c_size_t, [_i, _i]),

@@ -254,7 +254,8 @@ int dgs_key_bits(int width, int height, int F, int* tile_bits, int* subframe_bit
     return DGS_OK;
 }
 
-/* Shared implementation of dgs_blur_forward / dgs_blur_forward_hint / dgs_blur_forward_aa.
+/* Shared implementation of dgs_blur_forward / dgs_blur_forward_hint / dgs_blur_forward_aa / dgs_blur_forward_contrib.
+ *   contrib_wsum != NULL  the blend is the scoring kernel (contribution scores accumulated into contrib_wsum / _wmax).
  *   capacity_hint == 0  exact mode: the host waits for D after the scan stage (one synchronisation, like the
  *                       reference's rasterizer_impl.cu:287) and sizes the binning buffer from it.
  *   capacity_hint  > 0  speculative mode: the binning buffer is sized from the hint and every kernel of the view is
@@ -276,7 +277,8 @@ static int blur_forward_impl(
     int prefiltered, int use_sigmoid,
     float* out_color, float* out_depth, int* radii,
     float* out_blur, float blur_denominator,
-    int64_t capacity_hint, int64_t* num_rendered, int antialiasing, void* stream)
+    int64_t capacity_hint, int64_t* num_rendered, int antialiasing, void* stream,
+    unsigned long long* contrib_wsum = nullptr, uint32_t* contrib_wmax = nullptr)
 {
     cudaStream_t st = (cudaStream_t)stream;
     if (antialiasing != 0 && antialiasing != 1) return fail(DGS_ERR_INVALID_ARGUMENT, "antialiasing must be 0 or 1");
@@ -398,7 +400,7 @@ static int blur_forward_impl(
             }
         }
         if (F > 0 && pixels > 0) {
-            { StageTimer t(ST_RENDER_FWD, st, 1); launch_render_fwd(p, ranges, point_list, wmask, final_T, n_contrib, out_color, out_depth, st); }
+            { StageTimer t(ST_RENDER_FWD, st, 1); launch_render_fwd(p, ranges, point_list, wmask, final_T, n_contrib, out_color, out_depth, contrib_wsum, contrib_wmax, st); }
             if (out_blur) { StageTimer t(ST_BLUR_MEAN, st, 1); launch_blur_mean(out_color, F, 3 * pixels, blur_denominator, out_blur, st); }
         }
         DGS_CUDA(cudaGetLastError(), "forward launch");
@@ -483,6 +485,32 @@ int dgs_blur_forward_aa(
                              scale_modifier, rotations, cov3D_precomp, viewmatrix, projmatrix, campos, tan_fovx,
                              tan_fovy, z_near, z_far, prefiltered, use_sigmoid, out_color, out_depth, radii, out_blur,
                              blur_denominator, binning_capacity, num_rendered, antialiasing, stream);
+}
+
+int dgs_blur_forward_contrib(
+    dgs_alloc_fn geom_alloc, void* geom_ctx, dgs_alloc_fn binning_alloc, void* binning_ctx,
+    dgs_alloc_fn image_alloc, void* image_ctx,
+    int P, int F, int sh_degree, int sh_coeffs,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far,
+    int prefiltered, int use_sigmoid,
+    float* out_color, float* out_depth, int* radii,
+    float* out_blur, float blur_denominator,
+    int64_t binning_capacity, int64_t* num_rendered, int antialiasing,
+    uint64_t* contrib_wsum, uint32_t* contrib_wmax, void* stream)
+{
+    if (P > 0 && F > 0 && (!contrib_wsum || !contrib_wmax))
+        return fail(DGS_ERR_INVALID_ARGUMENT, "null contribution score array");
+    return blur_forward_impl(geom_alloc, geom_ctx, binning_alloc, binning_ctx, image_alloc, image_ctx, P, F, sh_degree,
+                             sh_coeffs, background, width, height, means3D, shs, colors_precomp, opacities, scales,
+                             scale_modifier, rotations, cov3D_precomp, viewmatrix, projmatrix, campos, tan_fovx,
+                             tan_fovy, z_near, z_far, prefiltered, use_sigmoid, out_color, out_depth, radii, out_blur,
+                             blur_denominator, binning_capacity, num_rendered, antialiasing, stream,
+                             (unsigned long long*)contrib_wsum, contrib_wmax);
 }
 
 size_t dgs_blur_forward_status_offset(int P, int F)

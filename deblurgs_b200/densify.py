@@ -172,6 +172,29 @@ class DensificationMixin:
         self._rebuild(src, int(src.numel()), keep_stats=True)
 
     @torch.no_grad()
+    def prune_by_contribution(self, scores, fraction=0.0, min_weight_max=0.0):
+        """Contribution-based pruning (LightGaussian's global significance, RadSplat's max weight): remove the
+        `fraction` of Gaussians with the lowest weight sum -- ties broken by index, lower first -- plus every
+        Gaussian whose largest blending weight is below `min_weight_max`.  `scores`: a `rasterizer.ContributionScores`
+        of this store (e.g. `CameraMotionModule.accumulate_contribution`).  One `prune_points` rebuild; returns the
+        boolean mask of the removed Gaussians."""
+        P = self._xyz.shape[0]
+        if scores.num_points != P:
+            raise ValueError("contribution scores hold %d Gaussians, the store %d" % (scores.num_points, P))
+        if not 0.0 <= fraction <= 1.0:
+            raise ValueError("fraction must be in [0, 1]")
+        dev = self._xyz.device
+        wsum = scores.wsum.to(dev)
+        mask = scores.weight_max.to(dev) < min_weight_max
+        n = int(math.floor(fraction * P))
+        if n > 0:
+            # stable sort of the exact integer sums: equal scores keep index order
+            order = torch.sort(wsum, stable=True).indices
+            mask[order[:n]] = True
+        self.prune_points(mask)
+        return mask
+
+    @torch.no_grad()
     def densification_postfix(self, new_xyz, new_features_dc, new_features_rest, new_opacities, new_scaling,
                               new_rotation):
         """Append new Gaussians (zero Adam moments) and reset the densification statistics."""

@@ -188,12 +188,27 @@ def all_reduce_densification_stats(stats):
     return stats
 
 
-def render_blurry_sharded(cmm, cam_idx, background, nu=None, grad_sink=None):
+@torch.no_grad()
+def all_reduce_contribution(scores):
+    """Make contribution scores identical on every rank, so that replicated Gaussian stores prune identically: with
+    `render_blurry_sharded` (or views split across ranks) each rank scores only what it rendered.  Weight sums add up,
+    maxima take the maximum (SUM on the int64 fixed-point sums, MAX on the float bits): exact, so the result equals
+    the scores of one process that rendered everything.  `scores`: rasterizer.ContributionScores, modified in place
+    and returned."""
+    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
+        return scores
+    dist.all_reduce(scores.wsum, op=dist.ReduceOp.SUM)
+    dist.all_reduce(scores.wmax, op=dist.ReduceOp.MAX)
+    return scores
+
+
+def render_blurry_sharded(cmm, cam_idx, background, nu=None, grad_sink=None, contrib=None):
     """Sub-frame-sharded blurry view: this rank renders its block of the F sub-frames of image
     `cam_idx`; returns (blurred [3,H,W] identical on every rank, local package, (start, stop)).
     Densification: the local package's statistics cover this rank's sub-frames only (already normalised by the
     view's full sub-frame count); call `all_reduce_densification_stats(pkg["densification"])` after backward and
-    before `add_densification_stats_blurry(pkg)` so that every rank accumulates the whole view."""
+    before `add_densification_stats_blurry(pkg)` so that every rank accumulates the whole view.  Likewise `contrib`
+    (rasterizer.ContributionScores) receives this rank's sub-frames only: `all_reduce_contribution` completes it."""
     from . import renderer
     rank, ws = world()
     view, proj, campos = cmm.get_trajectory_tensors(cam_idx, nu)
@@ -201,5 +216,5 @@ def render_blurry_sharded(cmm, cam_idx, background, nu=None, grad_sink=None):
     a, b = subframe_shard(F, rank, ws)
     pkg = renderer.render_blurry(view[a:b].contiguous(), proj[a:b].contiguous(), campos[a:b].contiguous(),
                                  cmm.original_cam[0], cmm.gaussians, background, blur_denominator=float(F),
-                                 grad_sink=grad_sink)
+                                 grad_sink=grad_sink, contrib=contrib)
     return all_reduce_sum(pkg["blurred"]), pkg, (a, b)

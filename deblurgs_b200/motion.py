@@ -296,9 +296,10 @@ class CameraMotionModule:
     def get_gt_image(self, idx):
         return getattr(self.original_cam[idx], "original_image", None)
 
-    def query(self, cam_idx, subframe_indice="all", post_process=None, background="random"):
+    def query(self, cam_idx, subframe_indice="all", post_process=None, background="random", contrib=None):
         """Render a blurry view. Same arguments and returned keys as the reference
-        (scene/motion.py:78-160): 'blurred', 'gt', 'subframes', 'depths', 'render_pkgs'."""
+        (scene/motion.py:78-160): 'blurred', 'gt', 'subframes', 'depths', 'render_pkgs'.
+        `contrib`: a `rasterizer.ContributionScores` the view's sub-frames add their contribution scores to."""
         assert self.gaussians is not None
         gaussians = self.gaussians
         if isinstance(background, str) and background == "random":
@@ -316,7 +317,7 @@ class CameraMotionModule:
                 subfr_idx = subframe_indice
             nu = nu[subfr_idx]
         view, proj, campos = self.get_trajectory_tensors(cam_idx, nu)
-        pkg = renderer.render_blurry(view, proj, campos, self.original_cam[0], gaussians, bg)
+        pkg = renderer.render_blurry(view, proj, campos, self.original_cam[0], gaussians, bg, contrib=contrib)
 
         blurred = pkg["blurred"]
         if post_process is not None:
@@ -328,3 +329,19 @@ class CameraMotionModule:
                        for s in range(F)]
         return {"blurred": blurred, "gt": self.get_gt_image(cam_idx), "subframes": pkg["render"],
                 "depths": pkg["depth"], "render_pkgs": render_pkgs, "batched": pkg}
+
+    @torch.no_grad()
+    def accumulate_contribution(self, background, cam_indices=None, scores=None):
+        """Contribution scores of the linked Gaussians over the training views: renders every sub-frame of the views
+        `cam_indices` (default: all) and returns `scores` (a new `rasterizer.ContributionScores` when None) with
+        their weights added.  Antialiasing follows the store, like every render, so the scores measure the opacity
+        that is actually blended.  Feed them to `gaussians.prune_by_contribution`."""
+        from .rasterizer import ContributionScores
+        assert self.gaussians is not None
+        if scores is None:
+            scores = ContributionScores(self.gaussians.get_xyz.shape[0], self.gaussians.get_xyz.device)
+        for idx in (range(len(self)) if cam_indices is None else cam_indices):
+            view, proj, campos = self.get_trajectory_tensors(idx)
+            renderer.render_blurry(view, proj, campos, self.original_cam[0], self.gaussians, background,
+                                   contrib=scores)
+        return scores

@@ -78,12 +78,53 @@ _last_scratch = None
 # the owner can read their status records.
 _ASYNC = None   # None, or {"capacity": int, "geoms": [(tensor, P, F), ...]}
 
+CONTRIB_SCALE = 1 << 26     # DGS_CONTRIB_SCALE: fixed-point scale of the contribution weight sums
+
+
+class ContributionScores:
+    """Per-Gaussian contribution scores, accumulated by every forward it is passed to (`contrib=`): over every pixel
+    of every rendered sub-frame where the blend used Gaussian g, with its blending weight w = alpha * T,
+      weight_sum[g] = sum of w   (LightGaussian's global significance; held as fixed point in `wsum`)
+      weight_max[g] = max of w   (RadSplat's pruning score; held as float bits in `wmax`).
+    Exact integer sums and maxima: the same bits on every run, batching and sharding of the same sub-frames.
+    The scores are those of the stored (with antialiasing: opacity * rho) opacity that is actually blended."""
+
+    def __init__(self, P, device):
+        self.wsum = torch.zeros(int(P), dtype=torch.int64, device=device)
+        self.wmax = torch.zeros(int(P), dtype=torch.int32, device=device)
+
+    @property
+    def num_points(self):
+        return self.wsum.shape[0]
+
+    @property
+    def weight_sum(self):
+        """float64 [P]: sum of the blending weights (each rounded to a multiple of 2^-26)."""
+        return self.wsum.double() / CONTRIB_SCALE
+
+    @property
+    def weight_max(self):
+        """float32 [P]: the largest blending weight."""
+        return self.wmax.view(torch.float32)
+
+    def reset(self):
+        self.wsum.zero_()
+        self.wmax.zero_()
+
+    def _check(self, P, device):
+        if self.num_points != P:
+            raise _lib.DgsError("ContributionScores holds %d Gaussians but the forward renders %d (the store changed "
+                                "size: make new scores after densify / prune)" % (self.num_points, P))
+        if self.wsum.device != device:
+            raise _lib.DgsError("ContributionScores live on %s, the forward runs on %s" % (self.wsum.device, device))
+
 
 def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                      viewmatrix, projmatrix, campos, bg, H, W, tanfovx, tanfovy, scale_modifier,
                      z_near, z_far, sh_degree, prefiltered, use_sigmoid, want_blur, blur_denominator, exact=False,
-                     antialiasing=False):
-    """Runs dgs_blur_forward_aa. viewmatrix/projmatrix [F,4,4], campos [F,3]."""
+                     antialiasing=False, contrib=None):
+    """Runs dgs_blur_forward_aa, or dgs_blur_forward_contrib with a `ContributionScores` to accumulate into.
+    viewmatrix/projmatrix [F,4,4], campos [F,3]."""
     lib = _lib.load()
     _require_cuda(means3D, "means3D")
     if means3D.dim() != 2 or means3D.shape[1] != 3:
@@ -91,6 +132,8 @@ def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, 
     dev = means3D.device
     P = means3D.shape[0]
     F = viewmatrix.shape[0]
+    if contrib is not None:
+        contrib._check(P, dev)
     M = sh.shape[1] if (sh is not None and sh.numel() != 0) else 0
     color = torch.empty((F, 3, H, W), dtype=torch.float32, device=dev)
     depth = torch.empty((F, 1, H, W), dtype=torch.float32, device=dev)
@@ -109,9 +152,7 @@ def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, 
     hint = 0 if (exact or os.environ.get("DGS_EXACT_BINNING") == "1") else _CAPACITY_HINT.get(shape_key, 0)
     if _ASYNC is not None:
         hint = int(_ASYNC["capacity"])
-    with torch.cuda.device(dev):
-        rc = lib.dgs_blur_forward_aa(
-            geom.cb, None, binning.cb, None, img.cb, None,
+    args = (geom.cb, None, binning.cb, None, img.cb, None,
             P, F, int(sh_degree), int(M),
             _lib.ptr(bg), int(W), int(H),
             _lib.ptr(means3D), _lib.ptr(sh), _lib.ptr(colors_precomp),
@@ -122,13 +163,18 @@ def _forward_batched(means3D, sh, colors_precomp, opacities, scales, rotations, 
             int(bool(prefiltered)), int(bool(use_sigmoid)),
             _lib.ptr(color), _lib.ptr(depth), _lib.ptr(radii),
             _lib.ptr(blur), float(blur_denominator),
-            int(hint), None if _ASYNC is not None else C.byref(num_rendered), int(bool(antialiasing)),
-            _stream_ptr(dev))
+            int(hint), None if _ASYNC is not None else C.byref(num_rendered), int(bool(antialiasing)))
+    entry = "dgs_blur_forward_aa" if contrib is None else "dgs_blur_forward_contrib"
+    with torch.cuda.device(dev):
+        if contrib is None:
+            rc = lib.dgs_blur_forward_aa(*args, _stream_ptr(dev))
+        else:
+            rc = lib.dgs_blur_forward_contrib(*args, _lib.ptr(contrib.wsum), _lib.ptr(contrib.wmax), _stream_ptr(dev))
     # drop the ctypes callbacks: they close over the _Buffer objects (a reference cycle), and a cycle
     # would keep hundreds of MB of state buffers alive until Python's cyclic GC runs, forcing the caching
     # allocator to cudaMalloc fresh blocks every step in the meantime
     geom.cb = binning.cb = img.cb = None
-    _lib.check(rc, "dgs_blur_forward_aa")
+    _lib.check(rc, entry)
     if _ASYNC is not None:
         _ASYNC["geoms"].append((geom.t, P, F))
         return color, depth, radii, blur, -1, geom.t, binning.t, img.t    # -1: number of duplicates unknown on the host
@@ -216,11 +262,11 @@ def _empty_like_input(t):
 
 class _RasterizeGaussians(torch.autograd.Function):
     """Single view. Same argument order, saved state and gradient tuple as the reference's
-    `_RasterizeGaussians` (diff_gaussian_rasterization/__init__.py:48-170), plus a trailing `antialiasing` flag."""
+    `_RasterizeGaussians` (diff_gaussian_rasterization/__init__.py:48-170), plus trailing `antialiasing` and `contrib`."""
 
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, antialiasing=False):
+                cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, antialiasing=False, contrib=None):
         rs = raster_settings
         ctx.set_materialize_grads(False)   # an unused output (depth) arrives as None, not as a zero-filled image
         means3D_c, sh_c, colors_c = _f32c(means3D), _f32c(sh), _f32c(colors_precomp)
@@ -232,7 +278,8 @@ class _RasterizeGaussians(torch.autograd.Function):
         color, depth, radii, _, num_rendered, geom, binning, img = _forward_batched(
             means3D_c, sh_c, colors_c, opac_c, scales_c, rot_c, cov_c, view_c, proj_c, campos_c, bg_c,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near,
-            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, False, 1.0, antialiasing=antialiasing)
+            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, False, 1.0, antialiasing=antialiasing,
+            contrib=contrib)
         ctx.raster_settings = rs
         ctx.num_rendered = num_rendered
         ctx.antialiasing = bool(antialiasing)
@@ -257,14 +304,16 @@ class _RasterizeGaussians(torch.autograd.Function):
         # reference order: means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
         # cov3Ds_precomp, viewmatrix, projmatrix, raster_settings
         return (dmeans3D, dmeans2D[0], dsh if sh.numel() != 0 else None, dcolors, dopacity, dscales, drot, dcov,
-                dview[0], dproj[0], None, None)
+                dview[0], dproj[0], None, None, None)
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                        viewmatrix, projmatrix, raster_settings, antialiasing=False):
-    """`antialiasing`: Mip-Splatting's screen-space filter (include/dgs_b200.h, dgs_blur_forward_aa)."""
+                        viewmatrix, projmatrix, raster_settings, antialiasing=False, contrib=None):
+    """`antialiasing`: Mip-Splatting's screen-space filter (include/dgs_b200.h, dgs_blur_forward_aa).
+    `contrib`: a `ContributionScores` the forward adds this view's contribution scores to."""
     return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                     cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, bool(antialiasing))
+                                     cov3Ds_precomp, viewmatrix, projmatrix, raster_settings, bool(antialiasing),
+                                     contrib)
 
 
 class _RasterizeBlurry(torch.autograd.Function):
@@ -276,7 +325,7 @@ class _RasterizeBlurry(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                 viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder=None,
-                antialiasing=False):
+                antialiasing=False, contrib=None):
         rs = raster_settings
         # outputs the loss does not use (typically the [F,3,H,W] / [F,1,H,W] stacks when only `blurred` is) arrive
         # as None in backward instead of zero-filled tensors the kernel would then have to read
@@ -290,7 +339,8 @@ class _RasterizeBlurry(torch.autograd.Function):
         color, depth, radii, blur, num_rendered, geom, binning, img = _forward_batched(
             means3D_c, sh_c, colors_c, opac_c, scales_c, rot_c, cov_c, view_c, proj_c, campos_c, bg_c,
             rs.image_height, rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near,
-            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing)
+            rs.z_far, rs.sh_degree, rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing,
+            contrib=contrib)
         ctx.raster_settings = rs
         ctx.num_rendered = num_rendered
         ctx.denom = denom
@@ -324,7 +374,7 @@ class _RasterizeBlurry(torch.autograd.Function):
             # the sub-frames still normalises its visible-count by all of them, train.py:193: 1 / len(render_pkgs))
             holder.fill(stats, ctx.denom)
         return (dmeans3D, dmeans2D, dsh if sh.numel() != 0 else None, dcolors, dopacity, dscales, drot, dcov,
-                dview, dproj, None, None, None, None, None)
+                dview, dproj, None, None, None, None, None, None)
 
 
 class _RenderStoreBlurry(torch.autograd.Function):
@@ -338,7 +388,7 @@ class _RenderStoreBlurry(torch.autograd.Function):
     @staticmethod
     def forward(ctx, xyz, f_dc, f_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix, campos,
                 raster_settings, blur_denominator, stats_holder, scale_lb, isotropic, grad_sink, n_ranges,
-                antialiasing=False):
+                antialiasing=False, contrib=None):
         lib = _lib.load()
         rs = raster_settings
         _require_cuda(xyz, "xyz")
@@ -363,7 +413,7 @@ class _RenderStoreBlurry(torch.autograd.Function):
         color, depth, radii, blur, num_rendered, geom, binning, img = _forward_batched(
             xyz_c, shs, None, opac, scales, rots, None, view_c, proj_c, campos_c, bg_c, rs.image_height,
             rs.image_width, rs.tanfovx, rs.tanfovy, rs.scale_modifier, rs.z_near, rs.z_far, rs.sh_degree,
-            rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing)
+            rs.prefiltered, rs.use_sigmoid, True, denom, antialiasing=antialiasing, contrib=contrib)
         ctx.raster_settings, ctx.num_rendered, ctx.denom = rs, num_rendered, denom
         ctx.antialiasing = bool(antialiasing)
         ctx.want_means2D = means2D is not None and means2D.requires_grad
@@ -424,16 +474,16 @@ class _RenderStoreBlurry(torch.autograd.Function):
             holder.fill(stats, ctx.denom)
         if sink is not None:
             sink.finish()
-            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 9
-        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 9
+            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 10
+        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 10
 
 
 def render_store_blurry(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix,
                         campos, raster_settings, blur_denominator=None, stats_holder=None, scale_lower_bound=0.0,
-                        isotropic=False, grad_sink=None, n_ranges=4, antialiasing=False):
+                        isotropic=False, grad_sink=None, n_ranges=4, antialiasing=False, contrib=None):
     return _RenderStoreBlurry.apply(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix,
                                     projmatrix, campos, raster_settings, blur_denominator, stats_holder,
-                                    scale_lower_bound, isotropic, grad_sink, n_ranges, bool(antialiasing))
+                                    scale_lower_bound, isotropic, grad_sink, n_ranges, bool(antialiasing), contrib)
 
 
 class DensificationStats:
@@ -461,24 +511,25 @@ class DensificationStats:
 
 def rasterize_blurry(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                      viewmatrix, projmatrix, campos, raster_settings, blur_denominator=None, stats_holder=None,
-                     antialiasing=False):
+                     antialiasing=False, contrib=None):
     empty = torch.Tensor([])
     return _RasterizeBlurry.apply(
         means3D, means2D, sh if sh is not None else empty,
         colors_precomp if colors_precomp is not None else empty, opacities,
         scales if scales is not None else empty, rotations if rotations is not None else empty,
         cov3Ds_precomp if cov3Ds_precomp is not None else empty,
-        viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder, bool(antialiasing))
+        viewmatrix, projmatrix, campos, raster_settings, blur_denominator, stats_holder, bool(antialiasing), contrib)
 
 
 class GaussianRasterizer(nn.Module):
-    """`antialiasing` is a constructor argument, not a settings field: GaussianRasterizationSettings keeps the
-    reference's 13 fields."""
+    """`antialiasing` and `contrib` (a `ContributionScores` every forward adds to) are constructor arguments, not
+    settings fields: GaussianRasterizationSettings keeps the reference's 13 fields."""
 
-    def __init__(self, raster_settings, antialiasing=False):
+    def __init__(self, raster_settings, antialiasing=False, contrib=None):
         super().__init__()
         self.raster_settings = raster_settings
         self.antialiasing = bool(antialiasing)
+        self.contrib = contrib
 
     def markVisible(self, positions, viewmatrix=None, projmatrix=None):
         """Frustum test. The reference reads `raster_settings.viewmatrix`, a field that no longer
@@ -522,4 +573,5 @@ class GaussianRasterizer(nn.Module):
             cov3D_precomp = torch.Tensor([])
 
         return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
-                                   cov3D_precomp, viewmatrix, projmatrix, raster_settings, self.antialiasing)
+                                   cov3D_precomp, viewmatrix, projmatrix, raster_settings, self.antialiasing,
+                                   self.contrib)

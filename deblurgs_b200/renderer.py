@@ -12,12 +12,13 @@ from .rasterizer import (DensificationStats, GaussianRasterizationSettings, Gaus
                          rasterize_blurry, render_store_blurry)
 
 
-def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=None, *_compat):
+def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=None, *_compat, contrib=None):
     """Render the scene from one camera. Background tensor (bg_color) must be on the GPU.
 
     Also tolerates the upstream-3DGS call form render(cam, pc, pipe, bg_color, ...): a third
     positional argument that is not a Tensor is taken to be `pipe` and ignored.
     Antialiasing follows `pc.antialiasing` (off when the store has no such attribute).
+    `contrib`: a `rasterizer.ContributionScores` this render adds its contribution scores to.
     """
     if not torch.is_tensor(bg_color):
         bg_color = scaling_modifier
@@ -48,7 +49,8 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
         prefiltered=False,
         debug=False,
     )
-    rasterizer = GaussianRasterizer(raster_settings=raster_settings, antialiasing=getattr(pc, "antialiasing", False))
+    rasterizer = GaussianRasterizer(raster_settings=raster_settings, antialiasing=getattr(pc, "antialiasing", False),
+                                    contrib=contrib)
 
     shs = None
     colors_precomp = None
@@ -77,14 +79,14 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
 
 
 def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, ref_cam, pc, bg_color,
-                  scaling_modifier=1.0, override_color=None, blur_denominator=None, grad_sink=None):
+                  scaling_modifier=1.0, override_color=None, blur_denominator=None, grad_sink=None, *, contrib=None):
     """Render all F sub-frames of a blurry view in one batched call.
 
     world_view_transforms / full_proj_transforms [F,4,4], camera_centers [F,3]: the MiniCam tensors of
     the sub-frames (e.g. from `pose.bezier_se3_poses`); `ref_cam` supplies image size and FoV.
     The Gaussian activations (pc.get_*) are evaluated once for the whole view, not once per sub-frame.
     Returns the reference's per-render dict with a leading sub-frame axis, plus "blurred".
-    Antialiasing follows `pc.antialiasing`, as in `render`.
+    Antialiasing follows `pc.antialiasing`, as in `render`; `contrib` as in `render`.
     """
     xyz = pc.get_xyz
     F = world_view_transforms.shape[0]
@@ -117,7 +119,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
             pc._xyz, pc._features_dc, pc._features_rest, pc._scaling, pc._rotation, pc._opacity, screenspace_points,
             world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats,
             getattr(pc, "scale_lower_bound", 0.0), getattr(pc, "use_isotropic", False), sink,
-            int(getattr(sink, "n_ranges", 4)), getattr(pc, "antialiasing", False))
+            int(getattr(sink, "n_ranges", 4)), getattr(pc, "antialiasing", False), contrib)
         return {"render": color, "depth": depth, "blurred": blurred, "viewspace_points": screenspace_points,
                 "visibility_filter": radii > 0, "radii": radii, "densification": stats}
     if hasattr(pc, "get_activated"):
@@ -131,7 +133,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
     color, depth, radii, blurred = rasterize_blurry(
         xyz, screenspace_points, shs, override_color, opacities, scales, rotations, None,
         world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats,
-        getattr(pc, "antialiasing", False))
+        getattr(pc, "antialiasing", False), contrib)
     return {"render": color,
             "depth": depth,
             "blurred": blurred,

@@ -22,9 +22,12 @@ scored the way DeblurGS is judged: the trained and the hidden scene rendered sha
 pose, PSNR / SSIM before and after training (refine.evaluate_views), at full size and at half resolution (a camera of
 W/2 x H/2 with the same field of view, scored against the full-size sharp truth averaged over 2x2 pixel boxes).
 --antialiasing renders both the hidden and the trained scene with the screen-space antialiasing filter.
+--prune-fraction f: at iteration --prune-at (default: half of --iters) every training view is swept for the
+contribution scores (CameraMotionModule.accumulate_contribution) and the fraction f of Gaussians with the lowest
+blending-weight sum is removed (prune_by_contribution); training then continues on the smaller store.
 
   python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000] [--lambda-dssim 0.2]
-                                        [--antialiasing]
+                                        [--antialiasing] [--prune-fraction 0.5 [--prune-at 100]]
 """
 import argparse
 import os
@@ -72,7 +75,11 @@ def main():
     ap.add_argument("--densify-every", type=int, default=100, help="0: never")
     ap.add_argument("--lambda-dssim", type=float, default=0.0, help="weight of the D-SSIM term (3DGS uses 0.2)")
     ap.add_argument("--antialiasing", action="store_true", help="screen-space antialiasing filter (Mip-Splatting)")
+    ap.add_argument("--prune-fraction", type=float, default=0.0,
+                    help="prune this fraction of Gaussians by contribution score (0: never)")
+    ap.add_argument("--prune-at", type=int, default=None, help="iteration of the contribution pruning (default iters/2)")
     args = ap.parse_args()
+    prune_at = args.iters // 2 if args.prune_at is None else args.prune_at
     if args.width % 2 or args.height % 2:
         raise SystemExit("--width and --height must be even (the half-resolution views average 2x2 pixel boxes)")
     dev = torch.device("cuda", 0)
@@ -130,7 +137,19 @@ def main():
 
     lam0, lam1 = 1e-3, 1e-5     # lambda_t_smooth_init / final (arguments/__init__.py:97-98)
     log, t0 = [], time.perf_counter()
+    t_prune, it_prune = None, 0
     for it in range(args.iters):
+        if args.prune_fraction > 0 and it == prune_at:
+            torch.cuda.synchronize()
+            t_prune, it_prune = time.perf_counter(), it
+            n_before = gauss.get_xyz.shape[0]
+            scores = cmm.accumulate_contribution(bg)
+            gauss.prune_by_contribution(scores, fraction=args.prune_fraction)
+            torch.cuda.synchronize()
+            print("iter %4d  contribution prune: %d -> %d Gaussians (sweep + prune %.1f ms); %.2f ms / iteration before"
+                  % (it, n_before, gauss.get_xyz.shape[0], 1e3 * (time.perf_counter() - t_prune),
+                     1e3 * (t_prune - t0) / max(it, 1)), flush=True)
+            t_prune = time.perf_counter()
         idx = it % args.views
         lam = lam0 * (lam1 / lam0) ** (it / max(args.iters - 1, 1))
         out = cmm.query(idx, "all", background=bg)
@@ -150,6 +169,9 @@ def main():
             print("iter %4d  loss %.5f" % log[-1], flush=True)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
+    if t_prune is not None:
+        print("%.2f ms / iteration after the contribution prune; %d Gaussians at the end"
+              % (1e3 * (time.perf_counter() - t_prune) / max(args.iters - it_prune, 1), gauss.get_xyz.shape[0]))
     print("%d iterations in %.2f s (%.2f ms / blurry view incl. optimizer); loss %.5f -> %.5f; "
           "densification: %d Gaussians seen, max screen radius %d px"
           % (args.iters, dt, 1e3 * dt / args.iters, log[0][1], log[-1][1], int((gauss.denom > 0).sum()),

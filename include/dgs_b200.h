@@ -228,6 +228,39 @@ int dgs_blur_backward_range_aa(
     float* dL_dviewmatrix, float* dL_dprojmatrix, float* densify_stats,
     int64_t g_begin, int64_t g_end, int stages, int antialiasing, void* stream);
 
+/*
+ * Contribution scores (DESIGN.md section 3).  dgs_blur_forward_aa plus, for every Gaussian g, over every pixel of every
+ * sub-frame where the blend actually used it, with its blending weight w = alpha * T (the weight of its colour term):
+ *   contrib_wsum[g] += sum of round(w * DGS_CONTRIB_SCALE)     (fixed point: at most 2^-27 error per blended pixel)
+ *   contrib_wmax[g]  = max(contrib_wmax[g], bits of max w)     (float bits: non-negative floats order like their bits)
+ * Both are device arrays of [P], ACCUMULATED into: zero them before the first call (wmax = 0 is the float 0).  Integer
+ * sums and maxima do not depend on the order of the additions, so the scores are the same bits on every run and for
+ * any batching of the sub-frames.  Images, depths, radii and every state buffer are exactly those of
+ * dgs_blur_forward_aa (a following dgs_blur_backward_range_aa is valid as usual).
+ * A speculative call (binning_capacity > 0) whose hint is too small blends empty lists first, which adds nothing;
+ * with num_rendered != NULL the blend is re-run with the exact size and adds the scores once, with num_rendered == NULL
+ * (nothing waited for) such an overflowed call adds nothing at all -- dgs_blur_forward_status reports it.
+ * NULL score pointers with P > 0 and F > 0, or an antialiasing value other than 0 / 1, fail with
+ * DGS_ERR_INVALID_ARGUMENT before any device work.
+ */
+#define DGS_CONTRIB_SCALE (1 << 26)
+int dgs_blur_forward_contrib(
+    dgs_alloc_fn geom_alloc, void* geom_ctx,
+    dgs_alloc_fn binning_alloc, void* binning_ctx,
+    dgs_alloc_fn image_alloc, void* image_ctx,
+    int P, int F, int sh_degree, int sh_coeffs,
+    const float* background, int width, int height,
+    const float* means3D, const float* shs, const float* colors_precomp,
+    const float* opacities, const float* scales, float scale_modifier,
+    const float* rotations, const float* cov3D_precomp,
+    const float* viewmatrix, const float* projmatrix, const float* campos,
+    float tan_fovx, float tan_fovy, float z_near, float z_far,
+    int prefiltered, int use_sigmoid,
+    float* out_color, float* out_depth, int* radii,
+    float* out_blur, float blur_denominator,
+    int64_t binning_capacity, int64_t* num_rendered, int antialiasing,
+    uint64_t* contrib_wsum, uint32_t* contrib_wmax, void* stream);
+
 /* Single-view pair: the reference's rasterize_gaussians / rasterize_gaussians_backward
  * (same argument meaning; F = 1 instance of the batched pair). */
 int dgs_forward(
