@@ -78,7 +78,11 @@ SIGNATURES = {
     "dgs_ssim_backward": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p]),
     "dgs_activate_forward": (_i, [_i, _i, _p, _p, _p, _p, _p, _f, _i, _p, _p, _p, _p, _p]),
     "dgs_activate_backward": (_i, [_i, _i, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
-    "dgs_adam_step": (_i, [_i, _p, _p, _p, _p, C.POINTER(_i64), C.POINTER(C.c_double), C.POINTER(_i64),
+    "dgs_activate_forward_filter3d": (_i, [_i, _i, _p, _p, _p, _p, _p, _f, _i, _p, _p, _p, _p, _p, _p]),
+    "dgs_activate_backward_filter3d": (_i, [_i, _i, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _f, _p,
+                                            _p]),
+    "dgs_filter3d_depth": (_i, [_i64, _p, _i, _p, _f, _f, _i, _i, _f, _p, _p]),
+    "dgs_adam_step":(_i, [_i, _p, _p, _p, _p, C.POINTER(_i64), C.POINTER(C.c_double), C.POINTER(_i64),
                            C.c_double, C.c_double, C.c_double, C.c_double, _p]),
     "dgs_rows_gather": (_i, [_i, _p, _p, C.POINTER(_i), C.POINTER(_i), _i64, _p, _p, _p]),
     "dgs_mark_visible": (_i, [_i, _p, _p, _p, _p, _p]),

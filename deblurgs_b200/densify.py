@@ -40,7 +40,9 @@ _GROUP_ATTR = {"xyz": "_xyz", "f_dc": "_features_dc", "f_rest": "_features_rest"
 
 class DensificationMixin:
     """Needs: the six raw parameter attributes, `optimizer` (param_groups named as in training_setup),
-    `get_scaling` / `get_opacity` / `get_xyz`, `scale_lower_bound`, and the statistics buffers."""
+    `get_scaling` / `get_opacity` / `get_xyz`, `scale_lower_bound`, and the statistics buffers; optionally `filter_3D`
+    (Mip-Splatting's 3-D filter), which every rebuild carries along.  The selection rules read the unfiltered getters,
+    as Mip-Splatting's do."""
 
     percent_dense = 0.01          # arguments/__init__.py:94
     alpha_lower_bound = 0.0       # arguments/__init__.py:68
@@ -112,6 +114,10 @@ class DensificationMixin:
         if keep_stats:
             items += [("stat", "xyz_gradient_accum", self.xyz_gradient_accum, 0), ("stat", "denom", self.denom, 0),
                       ("stat", "max_radii2D", self.max_radii2D.float(), 0)]
+        filter_3D = getattr(self, "filter_3D", None)
+        if filter_3D is not None:
+            # Mip-Splatting's 3-D filter: appended (clone / split) rows inherit their parent's value
+            items.append(("filter", "filter_3D", filter_3D, 0))
         outs = [torch.empty((n_out,) + tuple(t.shape[1:]), dtype=torch.float32, device=dev) for (_, _, t, _) in items]
         if dev.type == "cuda":
             lib = _lib.load()
@@ -155,6 +161,8 @@ class DensificationMixin:
                 g["params"][0] = param
             tensors[name] = param
         self._assign(tensors)
+        if filter_3D is not None:
+            self.filter_3D = new[("filter", "filter_3D")]
         if keep_stats:
             self.xyz_gradient_accum = new[("stat", "xyz_gradient_accum")]
             self.denom = new[("stat", "denom")]
@@ -197,11 +205,15 @@ class DensificationMixin:
     @torch.no_grad()
     def densification_postfix(self, new_xyz, new_features_dc, new_features_rest, new_opacities, new_scaling,
                               new_rotation):
-        """Append new Gaussians (zero Adam moments) and reset the densification statistics."""
+        """Append new Gaussians (zero Adam moments) and reset the densification statistics.  With the 3-D filter on,
+        the new Gaussians get a zero filter (unfiltered) until the next `CameraMotionModule.compute_3D_filter`."""
         self._assign(self.cat_tensors_to_optimizer({"xyz": new_xyz, "f_dc": new_features_dc,
                                                     "f_rest": new_features_rest, "opacity": new_opacities,
                                                     "scaling": new_scaling, "rotation": new_rotation}))
         P, dev = self._xyz.shape[0], self._xyz.device
+        filter_3D = getattr(self, "filter_3D", None)
+        if filter_3D is not None:
+            self.filter_3D = torch.cat((filter_3D, filter_3D.new_zeros((P - filter_3D.shape[0], 1))), dim=0)
         self.xyz_gradient_accum = torch.zeros((P, 1), device=dev)
         self.denom = torch.zeros((P, 1), device=dev)
         self.max_radii2D = torch.zeros(P, device=dev)
@@ -252,10 +264,16 @@ class DensificationMixin:
 
     @torch.no_grad()
     def reset_opacity(self, new_opacity=None):
-        """Cap every opacity at `new_opacity` (default 0.1) and zero its Adam moments (scene/gaussian_model.py:247-254)."""
+        """Cap every opacity at `new_opacity` (default 0.1) and zero its Adam moments (scene/gaussian_model.py:247-254).
+        With the 3-D filter on, the cap applies to the filtered opacity, as in Mip-Splatting's reset_opacity: the new
+        clamped opacity is min(o, cap / prod_i r_i), so that the filtered one is min(o prod_i r_i, cap)."""
         if new_opacity is None:
             lb = self.alpha_lower_bound
             new_opacity = lb + (1 - lb) * 0.1
         opac = self.get_opacity
-        capped = torch.min(opac, torch.ones_like(opac) * new_opacity).clamp(0.0, 1.0)
+        if getattr(self, "filter_3D", None) is not None:
+            r = self._filter_3D_ratios()
+            capped = torch.min(opac, new_opacity / (r[:, 0:1] * r[:, 1:2] * r[:, 2:3])).clamp(0.0, 1.0)
+        else:
+            capped = torch.min(opac, torch.ones_like(opac) * new_opacity).clamp(0.0, 1.0)
         self._assign(self.replace_tensor_to_optimizer(capped, "opacity"))

@@ -29,7 +29,10 @@ class BlurryViewGraph:
         step.check()                           # after a synchronisation: re-captures + replays if the capacity was exceeded
     `parameters` (default: the Gaussians' and the trajectory's) get their .grad from the captured backward.
     The store's `antialiasing` flag is read when the step is captured and is part of the graph: a replay after the flag
-    was changed raises DgsError (build a new BlurryViewGraph for the other setting) instead of rendering the old one."""
+    was changed raises DgsError (build a new BlurryViewGraph for the other setting) instead of rendering the old one.
+    So is the 3-D filter (`filter_3D`): whether it is on and which tensor holds it are fixed at capture, and a replay
+    after either changed raises.  Recomputing it in place (`CameraMotionModule.compute_3D_filter` on an unchanged
+    store) is what a replay sees: the graph reads the tensor's current values."""
 
     def __init__(self, cmm, cam_idx, background, gt_shape, lambda_t_smooth=0.0, parameters=None, pre_backward=None,
                  caller_owned_grads=(), capacity_margin=1.25, post_backward=None, render_fn=None,
@@ -54,6 +57,7 @@ class BlurryViewGraph:
         self.graph, self.loss, self.out, self.capacity = None, None, None, 0
         self.recaptures = 0
         self.antialiasing = self._store_antialiasing()
+        self.filter_3D_ptr = self._store_filter_3D()
         self._capture(None)
 
     # ------------------------------------------------------------------------------------------
@@ -73,6 +77,10 @@ class BlurryViewGraph:
 
     def _store_antialiasing(self):
         return bool(getattr(self.cmm.gaussians, "antialiasing", False))
+
+    def _store_filter_3D(self):
+        f = getattr(self.cmm.gaussians, "filter_3D", None)
+        return None if f is None else f.data_ptr()
 
     def _reset_grads(self):
         for p in self.params:
@@ -122,6 +130,11 @@ class BlurryViewGraph:
         if self._store_antialiasing() != self.antialiasing:
             raise _lib.DgsError("the store's antialiasing flag changed since this step was captured (captured with "
                                 "antialiasing=%s): build a new BlurryViewGraph for the new setting" % self.antialiasing)
+        if self._store_filter_3D() != self.filter_3D_ptr:
+            raise _lib.DgsError("the store's 3-D filter was %s since this step was captured: build a new BlurryViewGraph "
+                                "(an in-place compute_3D_filter keeps the graph valid)"
+                                % ("turned on" if self.filter_3D_ptr is None else
+                                   "turned off" if self._store_filter_3D() is None else "replaced"))
         self.graph.replay()
         for p, g in zip(self.params, self.grads):      # re-attach if someone replaced or cleared a .grad meanwhile
             if p.grad is not g:

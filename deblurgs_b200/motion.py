@@ -98,6 +98,8 @@ class GaussianParams(DensificationMixin):
         self.scale_lower_bound = scale_lower_bound
         self.use_isotropic = use_isotropic
         self.antialiasing = antialiasing   # screen-space antialiasing filter, read by renderer.render / render_blurry
+        # Mip-Splatting's 3-D smoothing filter [P,1] (CameraMotionModule.compute_3D_filter); None: off
+        self.filter_3D = None
         self.optimizer = None
         self.grad_sink = None      # optional dist.FlatGradBuffer.for_gaussians(self): gradients all-reduced under the backward
 
@@ -161,9 +163,10 @@ class GaussianParams(DensificationMixin):
 
     def get_activated(self):
         """(get_features, get_scaling, get_rotation, get_opacity) from ONE fused launch; what the batched
-        renderer reads once per blurry view."""
+        renderer reads once per blurry view.  With `filter_3D` set, the scaling and opacity are the filtered ones
+        (get_scaling_with_3D_filter / get_opacity_with_3D_filter)."""
         return activate_gaussians(self._features_dc, self._features_rest, self._scaling, self._rotation,
-                                  self._opacity, self.scale_lower_bound, self.use_isotropic)
+                                  self._opacity, self.scale_lower_bound, self.use_isotropic, self.filter_3D)
 
     @property
     def get_xyz(self):
@@ -186,6 +189,28 @@ class GaussianParams(DensificationMixin):
     @property
     def get_features(self):
         return torch.cat((self._features_dc, self._features_rest), dim=1)
+
+    # ---- Mip-Splatting's 3-D filter in torch (scene/gaussian_model.py get_*_with_3D_filter): what `renderer.render`
+    # reads, and the statement the fused kernel is tested against.  The opacity factor sqrt(det1 / det2) is written
+    # as the product of per-axis ratios s_i / s'_i, which does not underflow in fp32 for tiny scales.
+    @property
+    def get_scaling_with_3D_filter(self):
+        s = self.get_scaling
+        if self.filter_3D is None:
+            return s
+        return torch.sqrt(torch.square(s) + torch.square(self.filter_3D))
+
+    @property
+    def get_opacity_with_3D_filter(self):
+        o = self.get_opacity
+        if self.filter_3D is None:
+            return o
+        r = self._filter_3D_ratios()
+        return o * r[:, 0:1] * r[:, 1:2] * r[:, 2:3]
+
+    def _filter_3D_ratios(self):
+        s = self.get_scaling
+        return s / torch.sqrt(torch.square(s) + torch.square(self.filter_3D))
 
 
 class CameraMotionModule:
@@ -329,6 +354,26 @@ class CameraMotionModule:
                        for s in range(F)]
         return {"blurred": blurred, "gt": self.get_gt_image(cam_idx), "subframes": pkg["render"],
                 "depths": pkg["depth"], "render_pkgs": render_pkgs, "batched": pkg}
+
+    @torch.no_grad()
+    def compute_3D_filter(self, cam_indices=None):
+        """Mip-Splatting's compute_3D_filter over the sub-frame poses of the training views `cam_indices` (default:
+        all): sets and returns `gaussians.filter_3D` [P,1].  When the store already holds a filter of this size it is
+        overwritten in place, so that a captured `graph.BlurryViewGraph` replays with the new values."""
+        from .filter3d import SamplingDepth
+        assert self.gaussians is not None
+        g, ref = self.gaussians, self.original_cam[0]
+        xyz = g.get_xyz
+        depth = SamplingDepth(xyz.shape[0], xyz.device)
+        for idx in (range(len(self)) if cam_indices is None else cam_indices):
+            view, _, _ = self.get_trajectory_tensors(idx)
+            depth.add(xyz, view, ref.image_width, ref.image_height, ref.FoVx, ref.FoVy, g.z_near)
+        f = depth.filter_3D()
+        if g.filter_3D is not None and g.filter_3D.shape == f.shape and g.filter_3D.device == f.device:
+            g.filter_3D.copy_(f)
+        else:
+            g.filter_3D = f
+        return g.filter_3D
 
     @torch.no_grad()
     def accumulate_contribution(self, background, cam_indices=None, scores=None):

@@ -22,7 +22,8 @@ def _stream(dev):
 
 class _ActivateGaussians(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, features_dc, features_rest, scaling, rotation, opacity, scale_lower_bound, isotropic):
+    def forward(ctx, features_dc, features_rest, scaling, rotation, opacity, scale_lower_bound, isotropic,
+                filter3d=None):
         lib = _lib.load()
         if not scaling.is_cuda:
             raise _lib.DgsError("Gaussian parameters must be CUDA tensors: libdgs_b200 has no CPU path")
@@ -35,41 +36,57 @@ class _ActivateGaussians(torch.autograd.Function):
         scales = torch.empty((P, 3), dtype=torch.float32, device=dev)
         rots = torch.empty((P, 4), dtype=torch.float32, device=dev)
         opac = torch.empty((P, 1), dtype=torch.float32, device=dev)
+        filt = None if filter3d is None else filter3d.detach().float().contiguous()
+        if filt is not None and filt.numel() != P:
+            raise _lib.DgsError("filter_3D holds %d values, the store %d Gaussians" % (filt.numel(), P))
         with torch.cuda.device(dev):
-            rc = lib.dgs_activate_forward(P, M, _lib.ptr(dc), _lib.ptr(rest), _lib.ptr(sc), _lib.ptr(rot), _lib.ptr(op),
-                                          float(scale_lower_bound), int(bool(isotropic)), _lib.ptr(shs),
-                                          _lib.ptr(scales), _lib.ptr(rots), _lib.ptr(opac), _stream(dev))
+            if filt is None:
+                rc = lib.dgs_activate_forward(P, M, _lib.ptr(dc), _lib.ptr(rest), _lib.ptr(sc), _lib.ptr(rot),
+                                              _lib.ptr(op), float(scale_lower_bound), int(bool(isotropic)),
+                                              _lib.ptr(shs), _lib.ptr(scales), _lib.ptr(rots), _lib.ptr(opac),
+                                              _stream(dev))
+            else:
+                rc = lib.dgs_activate_forward_filter3d(P, M, _lib.ptr(dc), _lib.ptr(rest), _lib.ptr(sc), _lib.ptr(rot),
+                                                       _lib.ptr(op), float(scale_lower_bound), int(bool(isotropic)),
+                                                       _lib.ptr(shs), _lib.ptr(scales), _lib.ptr(rots), _lib.ptr(opac),
+                                                       filt.data_ptr(), _stream(dev))
         _lib.check(rc, "dgs_activate_forward")
         ctx.save_for_backward(sc, rot, op)
-        ctx.meta = (P, M, bool(isotropic), features_dc.shape, features_rest.shape)
+        ctx.filter3d = filt
+        ctx.meta = (P, M, bool(isotropic), features_dc.shape, features_rest.shape, float(scale_lower_bound))
         return shs, scales, rots, opac
 
     @staticmethod
     def backward(ctx, dshs, dscales, drots, dopac):
         lib = _lib.load()
         sc, rot, op = ctx.saved_tensors
-        P, M, isotropic, dc_shape, rest_shape = ctx.meta
+        P, M, isotropic, dc_shape, rest_shape, lb = ctx.meta
         dev = sc.device
         f = lambda t: None if t is None else t.float().contiguous()
         dshs, dscales, drots, dopac = f(dshs), f(dscales), f(drots), f(dopac)
         ddc = torch.empty(dc_shape, dtype=torch.float32, device=dev)
         drest = torch.empty(rest_shape, dtype=torch.float32, device=dev)
         dsc, drot, dop = torch.empty_like(sc), torch.empty_like(rot), torch.empty_like(op)
+        args = (P, M, _lib.ptr(sc), _lib.ptr(rot), _lib.ptr(op), int(isotropic), _lib.ptr(dshs), _lib.ptr(dscales),
+                _lib.ptr(drots), _lib.ptr(dopac), _lib.ptr(ddc), _lib.ptr(drest), _lib.ptr(dsc), _lib.ptr(drot),
+                _lib.ptr(dop))
         with torch.cuda.device(dev):
-            rc = lib.dgs_activate_backward(P, M, _lib.ptr(sc), _lib.ptr(rot), _lib.ptr(op), int(isotropic),
-                                           _lib.ptr(dshs), _lib.ptr(dscales), _lib.ptr(drots), _lib.ptr(dopac),
-                                           _lib.ptr(ddc), _lib.ptr(drest), _lib.ptr(dsc), _lib.ptr(drot),
-                                           _lib.ptr(dop), _stream(dev))
+            if ctx.filter3d is None:
+                rc = lib.dgs_activate_backward(*args, _stream(dev))
+            else:
+                rc = lib.dgs_activate_backward_filter3d(*args, lb, ctx.filter3d.data_ptr(), _stream(dev))
         _lib.check(rc, "dgs_activate_backward")
-        return ddc, drest, dsc, drot, dop, None, None
+        return ddc, drest, dsc, drot, dop, None, None, None
 
 
 def activate_gaussians(features_dc, features_rest, scaling, rotation, opacity, scale_lower_bound=0.0,
-                       isotropic=False):
+                       isotropic=False, filter3d=None):
     """(get_features [P,M,3], get_scaling [P,3], get_rotation [P,4], get_opacity [P,1]) of the reference's
-    GaussianModel in one launch, differentiable with respect to the five raw parameter tensors."""
+    GaussianModel in one launch, differentiable with respect to the five raw parameter tensors.
+    `filter3d` [P,1]: Mip-Splatting's 3-D smoothing filter (a constant without gradient); scales and opacities are
+    then those of get_scaling_with_3D_filter / get_opacity_with_3D_filter (include/dgs_b200.h)."""
     return _ActivateGaussians.apply(features_dc, features_rest, scaling, rotation, opacity, scale_lower_bound,
-                                    isotropic)
+                                    isotropic, filter3d)
 
 
 class FusedAdam:

@@ -388,7 +388,7 @@ class _RenderStoreBlurry(torch.autograd.Function):
     @staticmethod
     def forward(ctx, xyz, f_dc, f_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix, campos,
                 raster_settings, blur_denominator, stats_holder, scale_lb, isotropic, grad_sink, n_ranges,
-                antialiasing=False, contrib=None):
+                antialiasing=False, contrib=None, filter3d=None):
         lib = _lib.load()
         rs = raster_settings
         _require_cuda(xyz, "xyz")
@@ -401,11 +401,18 @@ class _RenderStoreBlurry(torch.autograd.Function):
         f32 = dict(dtype=torch.float32, device=dev)
         shs, scales = torch.empty((P, M, 3), **f32), torch.empty((P, 3), **f32)
         rots, opac = torch.empty((P, 4), **f32), torch.empty((P, 1), **f32)
+        filt = None if filter3d is None else _f32c(filter3d.detach())
+        if filt is not None and filt.numel() != P:
+            raise _lib.DgsError("filter_3D holds %d values, the store %d Gaussians" % (filt.numel(), P))
         if P > 0:
             with torch.cuda.device(dev):
-                rc = lib.dgs_activate_forward(P, M, _lib.ptr(dc_c), _lib.ptr(rest_c), _lib.ptr(sc_c), _lib.ptr(rot_c),
-                                              _lib.ptr(op_c), float(scale_lb), int(bool(isotropic)), _lib.ptr(shs),
-                                              _lib.ptr(scales), _lib.ptr(rots), _lib.ptr(opac), _stream_ptr(dev))
+                args = (P, M, _lib.ptr(dc_c), _lib.ptr(rest_c), _lib.ptr(sc_c), _lib.ptr(rot_c), _lib.ptr(op_c),
+                        float(scale_lb), int(bool(isotropic)), _lib.ptr(shs), _lib.ptr(scales), _lib.ptr(rots),
+                        _lib.ptr(opac))
+                if filt is None:
+                    rc = lib.dgs_activate_forward(*args, _stream_ptr(dev))
+                else:
+                    rc = lib.dgs_activate_forward_filter3d(*args, filt.data_ptr(), _stream_ptr(dev))
             _lib.check(rc, "dgs_activate_forward")
         view_c, proj_c, campos_c, bg_c = _f32c(viewmatrix), _f32c(projmatrix), _f32c(campos), _f32c(rs.bg)
         F = view_c.shape[0]
@@ -418,7 +425,8 @@ class _RenderStoreBlurry(torch.autograd.Function):
         ctx.antialiasing = bool(antialiasing)
         ctx.want_means2D = means2D is not None and means2D.requires_grad
         ctx.stats_holder, ctx.sink, ctx.n_ranges = stats_holder, grad_sink, max(1, int(n_ranges))
-        ctx.meta = (M, bool(isotropic), f_dc.shape, f_rest.shape)
+        ctx.meta = (M, bool(isotropic), f_dc.shape, f_rest.shape, float(scale_lb))
+        ctx.filter3d = filt
         ctx.save_for_backward(xyz_c, sc_c, rot_c, op_c, shs, scales, rots, opac, radii, geom, binning, img, view_c,
                               proj_c, campos_c, bg_c)
         ctx.mark_non_differentiable(radii)
@@ -429,7 +437,8 @@ class _RenderStoreBlurry(torch.autograd.Function):
         lib = _lib.load()
         rs = ctx.raster_settings
         (xyz, sc, rot, op, shs, scales, rots, opac, radii, geom, binning, img, view, proj, campos, bg) = ctx.saved_tensors
-        M, isotropic, dc_shape, rest_shape = ctx.meta
+        M, isotropic, dc_shape, rest_shape, scale_lb = ctx.meta
+        filt = ctx.filter3d
         P, F, dev = xyz.shape[0], view.shape[0], xyz.device
         f32 = dict(dtype=torch.float32, device=dev)
         gc = _f32c(grad_color) if grad_color is not None else None
@@ -455,11 +464,14 @@ class _RenderStoreBlurry(torch.autograd.Function):
         def after_range(g0, g1, _out):
             rows = g1 - g0
             o = lambda t, w: t.data_ptr() + g0 * w * 4
-            with torch.cuda.device(dev):
-                rc = lib.dgs_activate_backward(
-                    rows, M, o(sc, 3), o(rot, 4), o(op, 1), int(isotropic), o(dsh, 3 * M), o(dscales, 3), o(drots, 4),
+            args = (rows, M, o(sc, 3), o(rot, 4), o(op, 1), int(isotropic), o(dsh, 3 * M), o(dscales, 3), o(drots, 4),
                     o(dopac, 1), o(ddc, 3), o(drest, 3 * (M - 1)) if M > 1 else None, o(dsc, 3), o(drot_raw, 4),
-                    o(dop_raw, 1), st)
+                    o(dop_raw, 1))
+            with torch.cuda.device(dev):
+                if filt is None:
+                    rc = lib.dgs_activate_backward(*args, st)
+                else:
+                    rc = lib.dgs_activate_backward_filter3d(*args, scale_lb, o(filt, 1), st)
             _lib.check(rc, "dgs_activate_backward")
             if sink is not None:
                 sink.rows_done(g0, g1)
@@ -474,16 +486,18 @@ class _RenderStoreBlurry(torch.autograd.Function):
             holder.fill(stats, ctx.denom)
         if sink is not None:
             sink.finish()
-            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 10
-        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 10
+            return (None, None, None, None, None, None, dmeans2D, dview, dproj) + (None,) * 11
+        return (dxyz, ddc, drest, dsc, drot_raw, dop_raw, dmeans2D, dview, dproj) + (None,) * 11
 
 
 def render_store_blurry(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix, projmatrix,
                         campos, raster_settings, blur_denominator=None, stats_holder=None, scale_lower_bound=0.0,
-                        isotropic=False, grad_sink=None, n_ranges=4, antialiasing=False, contrib=None):
+                        isotropic=False, grad_sink=None, n_ranges=4, antialiasing=False, contrib=None, filter3d=None):
+    """`filter3d` [P,1]: Mip-Splatting's 3-D smoothing filter applied in the fused activations (params.activate_gaussians)."""
     return _RenderStoreBlurry.apply(xyz, features_dc, features_rest, scaling, rotation, opacity, means2D, viewmatrix,
                                     projmatrix, campos, raster_settings, blur_denominator, stats_holder,
-                                    scale_lower_bound, isotropic, grad_sink, n_ranges, bool(antialiasing), contrib)
+                                    scale_lower_bound, isotropic, grad_sink, n_ranges, bool(antialiasing), contrib,
+                                    filter3d)
 
 
 class DensificationStats:

@@ -17,7 +17,8 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
 
     Also tolerates the upstream-3DGS call form render(cam, pc, pipe, bg_color, ...): a third
     positional argument that is not a Tensor is taken to be `pipe` and ignored.
-    Antialiasing follows `pc.antialiasing` (off when the store has no such attribute).
+    Antialiasing follows `pc.antialiasing` (off when the store has no such attribute).  With `pc.filter_3D` set, the
+    scales and opacities are Mip-Splatting's filtered ones (`get_scaling_with_3D_filter` / `get_opacity_with_3D_filter`).
     `contrib`: a `rasterizer.ContributionScores` this render adds its contribution scores to.
     """
     if not torch.is_tensor(bg_color):
@@ -59,13 +60,17 @@ def render(viewpoint_camera, pc, bg_color, scaling_modifier=1.0, override_color=
     else:
         colors_precomp = override_color
 
+    if getattr(pc, "filter_3D", None) is not None:
+        opacities, scales = pc.get_opacity_with_3D_filter, pc.get_scaling_with_3D_filter
+    else:
+        opacities, scales = pc.get_opacity, pc.get_scaling
     rendered_image, rendered_depth, radii = rasterizer(
         means3D=pc.get_xyz,
         means2D=screenspace_points,
         shs=shs,
         colors_precomp=colors_precomp,
-        opacities=pc.get_opacity,
-        scales=pc.get_scaling,
+        opacities=opacities,
+        scales=scales,
         rotations=pc.get_rotation,
         cov3D_precomp=None,
         viewmatrix=viewpoint_camera.world_view_transform,
@@ -86,7 +91,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
     the sub-frames (e.g. from `pose.bezier_se3_poses`); `ref_cam` supplies image size and FoV.
     The Gaussian activations (pc.get_*) are evaluated once for the whole view, not once per sub-frame.
     Returns the reference's per-render dict with a leading sub-frame axis, plus "blurred".
-    Antialiasing follows `pc.antialiasing`, as in `render`; `contrib` as in `render`.
+    Antialiasing, the 3-D filter (`pc.filter_3D`) and `contrib` as in `render`.
     """
     xyz = pc.get_xyz
     F = world_view_transforms.shape[0]
@@ -112,6 +117,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
     )
     stats = DensificationStats()   # filled by the backward pass
     sink = grad_sink if grad_sink is not None else getattr(pc, "grad_sink", None)
+    filter3d = getattr(pc, "filter_3D", None)
     if sink is not None and override_color is None and hasattr(pc, "_features_rest"):
         # parameter store + gradient sink (dist.FlatGradBuffer): activations, render and a range-by-range backward in one
         # autograd node, so that the all-reduce of finished rows overlaps the rest of the backward
@@ -119,7 +125,7 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
             pc._xyz, pc._features_dc, pc._features_rest, pc._scaling, pc._rotation, pc._opacity, screenspace_points,
             world_view_transforms, full_proj_transforms, camera_centers, raster_settings, blur_denominator, stats,
             getattr(pc, "scale_lower_bound", 0.0), getattr(pc, "use_isotropic", False), sink,
-            int(getattr(sink, "n_ranges", 4)), getattr(pc, "antialiasing", False), contrib)
+            int(getattr(sink, "n_ranges", 4)), getattr(pc, "antialiasing", False), contrib, filter3d)
         return {"render": color, "depth": depth, "blurred": blurred, "viewspace_points": screenspace_points,
                 "visibility_filter": radii > 0, "radii": radii, "densification": stats}
     if hasattr(pc, "get_activated"):
@@ -128,6 +134,8 @@ def render_blurry(world_view_transforms, full_proj_transforms, camera_centers, r
     else:
         # any object with the reference's GaussianModel getters
         shs, scales, rotations, opacities = pc.get_features, pc.get_scaling, pc.get_rotation, pc.get_opacity
+        if filter3d is not None:
+            scales, opacities = pc.get_scaling_with_3D_filter, pc.get_opacity_with_3D_filter
     if override_color is not None:
         shs = None
     color, depth, radii, blurred = rasterize_blurry(

@@ -25,9 +25,14 @@ W/2 x H/2 with the same field of view, scored against the full-size sharp truth 
 --prune-fraction f: at iteration --prune-at (default: half of --iters) every training view is swept for the
 contribution scores (CameraMotionModule.accumulate_contribution) and the fraction f of Gaussians with the lowest
 blending-weight sum is removed (prune_by_contribution); training then continues on the smaller store.
+--filter3d: Mip-Splatting's 3-D smoothing filter on the trained store, computed from the sub-frame poses of every
+training view after initialisation, every --filter3d-every iterations and after each densify round.  The views are
+also scored at double size (a camera of 2W x 2H with the same field of view, against the hidden scene rendered sharp
+at that size without the filter): the zoom-in case the filter is for.
 
   python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000] [--lambda-dssim 0.2]
                                         [--antialiasing] [--prune-fraction 0.5 [--prune-at 100]]
+                                        [--filter3d [--filter3d-every 100]]
 """
 import argparse
 import os
@@ -78,6 +83,8 @@ def main():
     ap.add_argument("--prune-fraction", type=float, default=0.0,
                     help="prune this fraction of Gaussians by contribution score (0: never)")
     ap.add_argument("--prune-at", type=int, default=None, help="iteration of the contribution pruning (default iters/2)")
+    ap.add_argument("--filter3d", action="store_true", help="3-D smoothing filter on the trained store (Mip-Splatting)")
+    ap.add_argument("--filter3d-every", type=int, default=100, help="recompute the 3-D filter every N iterations")
     args = ap.parse_args()
     prune_at = args.iters // 2 if args.prune_at is None else args.prune_at
     if args.width % 2 or args.height % 2:
@@ -116,7 +123,8 @@ def main():
                                rotation_lr=0.001)
     # mid-trajectory camera pose of every view -> (c2w rotation, camera position), as COLMAP would give them
     half_cam = types.SimpleNamespace(width=cam.width // 2, height=cam.height // 2, fovx=cam.fovx, fovy=cam.fovy)
-    mid_R, mid_t, sharp, sharp_half = [], [], [], []
+    double_cam = types.SimpleNamespace(width=cam.width * 2, height=cam.height * 2, fovx=cam.fovx, fovy=cam.fovy)
+    mid_R, mid_t, sharp, sharp_half, sharp_double = [], [], [], [], []
     for t in true_traj:
         view, proj, campos = bezier_se3_poses(t.ctrl_trans, t.ctrl_rot, torch.tensor([0.5], device=dev),
                                               cams[0].projection_matrix)
@@ -129,10 +137,16 @@ def main():
         # the same pose and field of view at half the resolution, scored against the truth box-filtered to that size
         box = torch.nn.functional.avg_pool2d(v.original_image[None], 2)[0]
         sharp_half.append(SharpView(half_cam, view[0], proj[0], campos[0], box))
-    before, before_half = evaluate_views(sharp, gauss, bg), evaluate_views(sharp_half, gauss, bg)
+        with torch.no_grad():     # zoom-in: the same pose and field of view at twice the resolution
+            v2 = SharpView(double_cam, view[0], proj[0], campos[0], None)
+            v2.original_image = renderer.render(v2, truth, bg)["render"].clamp(0.0, 1.0)
+        sharp_double.append(v2)
     cmm = CameraMotionModule.from_poses(cams, torch.stack(mid_R), torch.stack(mid_t), curve_order=order,
                                         num_subframes=F)
     cmm.link_gaussian(gauss)
+    if args.filter3d:
+        cmm.compute_3D_filter()
+    before, before_half, before_double = (evaluate_views(v, gauss, bg) for v in (sharp, sharp_half, sharp_double))
     cmm.add_training_setup(gauss, {"curve_rot": 2e-4, "curve_trans": 2e-3, "curve_alignment": 0.0})
 
     lam0, lam1 = 1e-3, 1e-5     # lambda_t_smooth_init / final (arguments/__init__.py:97-98)
@@ -164,6 +178,10 @@ def main():
             n_before = gauss.get_xyz.shape[0]
             gauss.densify_and_prune(max_grad=2e-4, extent=5.0)       # train.py:195-196
             print("iter %4d  densify/prune: %d -> %d Gaussians" % (it, n_before, gauss.get_xyz.shape[0]), flush=True)
+            if args.filter3d:
+                cmm.compute_3D_filter()
+        elif args.filter3d and args.filter3d_every and it > 0 and it % args.filter3d_every == 0:
+            cmm.compute_3D_filter()
         if it % max(args.iters // 10, 1) == 0 or it == args.iters - 1:
             log.append((it, float(loss.detach())))
             print("iter %4d  loss %.5f" % log[-1], flush=True)
@@ -176,12 +194,13 @@ def main():
           "densification: %d Gaussians seen, max screen radius %d px"
           % (args.iters, dt, 1e3 * dt / args.iters, log[0][1], log[-1][1], int((gauss.denom > 0).sum()),
              int(gauss.max_radii2D.max())))
-    after, after_half = evaluate_views(sharp, gauss, bg), evaluate_views(sharp_half, gauss, bg)
+    after, after_half, after_double = (evaluate_views(v, gauss, bg) for v in (sharp, sharp_half, sharp_double))
     for label, b, a in (("full size %dx%d" % (cam.width, cam.height), before, after),
-                        ("half size %dx%d" % (half_cam.width, half_cam.height), before_half, after_half)):
-        print("sharp mid-exposure views vs the hidden scene, %s, antialiasing %s: PSNR %.2f -> %.2f dB, SSIM %.4f -> %.4f"
-              % (label, "on" if args.antialiasing else "off", b["psnr_mean"], a["psnr_mean"], b["ssim_mean"],
-                 a["ssim_mean"]))
+                        ("half size %dx%d" % (half_cam.width, half_cam.height), before_half, after_half),
+                        ("double size %dx%d" % (double_cam.width, double_cam.height), before_double, after_double)):
+        print("sharp mid-exposure views vs the hidden scene, %s, antialiasing %s, 3-D filter %s: PSNR %.2f -> %.2f dB, "
+              "SSIM %.4f -> %.4f" % (label, "on" if args.antialiasing else "off", "on" if args.filter3d else "off",
+                                     b["psnr_mean"], a["psnr_mean"], b["ssim_mean"], a["ssim_mean"]))
     assert log[-1][1] < 0.8 * log[0][1], "training did not reduce the loss"
 
 

@@ -433,6 +433,40 @@ int dgs_activate_backward(int P, int sh_coeffs, const float* scaling, const floa
                           float* dL_dscaling, float* dL_drotation, float* dL_dopacity, void* stream);
 
 /*
+ * Mip-Splatting's 3-D smoothing filter (Yu et al., CVPR 2024; reference: mip-splatting scene/gaussian_model.py).
+ *
+ * dgs_filter3d_depth restates the sweep of `compute_3D_filter` for n_cams cameras that share one set of intrinsics:
+ * viewmatrices [n_cams, 16] are world_view_transform (row-vector layout, p = [x, 1] . V).  For every Gaussian and
+ * camera, with z = p.z, z' = max(z, 0.001), u = p.x / z' * focal_x + width / 2, v = p.y / z' * focal_y + height / 2,
+ * the camera sees the Gaussian iff z > z_near and -0.15 width <= u <= 1.15 width and -0.15 height <= v <= 1.15 height.
+ * min_depth [P] (device, initialised by the caller, e.g. to +inf) is min-combined with the smallest z of the cameras
+ * that see each Gaussian.  A float min is exact, so successive calls compose over views and camera chunks and the
+ * result is bit-identical for any order or split of the same cameras.  The finalisation (filter = d_min / max focal
+ * * sqrt(0.2), unseen Gaussians at the largest finite d_min) is the caller's (deblurgs_b200/filter3d.py).
+ * Rejected before any device work: P < 0, n_cams < 0, a focal length or image size <= 0, and NULL pointers when
+ * P > 0 and n_cams > 0.
+ *
+ * dgs_activate_forward_filter3d: dgs_activate_forward with the filter of `get_scaling_with_3D_filter` /
+ * `get_opacity_with_3D_filter` applied, f = filter3d[g] (device, [P], a constant without gradient):
+ *   scales'_i = sqrt(s_i^2 + f^2),  opacity' = clamp(opacity, 0, 1) * r_0 * r_1 * r_2,  r_i = s_i / scales'_i,
+ * where s = exp(scaling) + scale_lower_bound.  The product of per-axis ratios equals Mip-Splatting's
+ * sqrt(det1 / det2) and does not underflow for s < ~1e-7 as prod(s_i^2) does in fp32.
+ * dgs_activate_backward_filter3d is its chain rule; it needs the forward's scale_lower_bound (the plain backward
+ * does not).  A NULL filter3d is rejected.  The plain entry points are the same implementation without the filter.
+ */
+int dgs_filter3d_depth(int64_t P, const float* means3D, int n_cams, const float* viewmatrices, float focal_x,
+                       float focal_y, int width, int height, float z_near, float* min_depth, void* stream);
+int dgs_activate_forward_filter3d(int P, int sh_coeffs, const float* features_dc, const float* features_rest,
+                                  const float* scaling, const float* rotation, const float* opacity,
+                                  float scale_lower_bound, int isotropic, float* shs, float* scales, float* rotations,
+                                  float* opacities, const float* filter3d, void* stream);
+int dgs_activate_backward_filter3d(int P, int sh_coeffs, const float* scaling, const float* rotation,
+                                   const float* opacity, int isotropic, const float* dL_dshs, const float* dL_dscales,
+                                   const float* dL_drotations, const float* dL_dopacities, float* dL_dfeatures_dc,
+                                   float* dL_dfeatures_rest, float* dL_dscaling, float* dL_drotation,
+                                   float* dL_dopacity, float scale_lower_bound, const float* filter3d, void* stream);
+
+/*
  * One Adam step over up to DGS_ADAM_MAX_TENSORS parameter tensors in a single launch: the reference's
  * `torch.optim.Adam(l, lr=0.0, eps=1e-15)` with one parameter per group and per-group learning rates
  * (scene/gaussian_model.py:175-190, train.py:204-208; amsgrad / weight decay / maximize off).
