@@ -85,6 +85,10 @@ SIGNATURES = {
     "dgs_adam_step":(_i, [_i, _p, _p, _p, _p, C.POINTER(_i64), C.POINTER(C.c_double), C.POINTER(_i64),
                            C.c_double, C.c_double, C.c_double, C.c_double, _p]),
     "dgs_rows_gather": (_i, [_i, _p, _p, C.POINTER(_i), C.POINTER(_i), _i64, _p, _p, _p]),
+    "dgs_mcmc_relocate_scratch_bytes": (C.c_size_t, [_i64]),
+    "dgs_mcmc_relocate": (_i, [_i, _p, C.POINTER(_i), C.POINTER(_i), _i64, _p, _p, _p, _f, _i, _p, _p]),
+    "dgs_mcmc_noise": (_i, [_i64, _p, _p, _p, _p, _f, _i, _f, _f, _f, C.c_uint64, _i64, _p]),
+    "dgs_debug_mcmc_normals": (_i, [_i64, C.c_uint64, _i64, _p, _p]),
     "dgs_mark_visible": (_i, [_i, _p, _p, _p, _p, _p]),
     "dgs_knn_scratch_bytes": (C.c_size_t, [_i]),
     "dgs_knn_mean_dist2": (_i, [_i, _p, _p, _p, _p]),

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libdgs_b200.so")
 SOURCES = ["dgs_forward.cu", "dgs_backward.cu", "dgs_binning.cu", "dgs_api.cu", "dgs_pose.cu", "dgs_knn.cu", "dgs_loss.cu", "dgs_params.cu",
-           "dgs_ssim.cu"]
+           "dgs_ssim.cu", "dgs_mcmc.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-gencode", "arch=compute_100a,code=sm_100a",
          "-lineinfo", "-I" + os.path.join(ROOT, "include"), "-I" + CSRC]

@@ -14,6 +14,10 @@ instead of the reference's append followed by a prune.  The selection rules are 
 With CPU tensors (unit tests of the semantics) the same plan is executed with torch indexing.  The per-step part --
 accumulating the statistics these rounds consume -- is fused into the backward kernel (`DensificationStats`).
 The WHEN (thresholds, schedules) remains the caller's policy, as in the reference's train.py:188-199.
+
+The 3DGS-MCMC alternative (`relocate_gs`, `add_new_gs`; mcmc.py) reads no gradient statistics: dead Gaussians are
+moved onto live ones drawn by opacity, in place (`dgs_mcmc_relocate`), and the store grows by a bounded fraction per
+round up to a cap.
 """
 import ctypes as C
 import math
@@ -261,6 +265,94 @@ class DensificationMixin:
         self.densify_and_split(grads, max_grad, extent, generator=generator)
         min_opacity = self.alpha_lower_bound + (1 - self.alpha_lower_bound) * 0.005
         self.prune_points((self.get_opacity < min_opacity).squeeze(-1))
+
+    # ---- 3DGS-MCMC (Kheradmand et al., NeurIPS 2024): relocation and growth --------------------------------------
+    @torch.no_grad()
+    def _relocate(self, dst, src):
+        """In place: row dst[r] of every per-Gaussian tensor becomes a copy of row src[r]; the opacity and scale of
+        every source are split between it and its copies (mcmc.relocation_values); the Adam moments and the
+        densification statistics of the source and destination rows are zeroed.  Every tensor keeps its identity and
+        storage.  Precondition: dst rows distinct and disjoint from the src rows.  One `dgs_mcmc_relocate` on the GPU."""
+        from . import mcmc
+        self._ensure_stats()
+        P, dev = self._xyz.shape[0], self._xyz.device
+        ratio = mcmc.relocation_ratio(src, P)
+        groups = {g["name"]: g for g in self.optimizer.param_groups if g["name"] in _GROUP_ATTR}
+        kind_of = {"opacity": 1, "scaling": 2}      # DGS_RELOCATE_OPACITY / _SCALING; parameters otherwise copied (0)
+        items = []                                   # (tensor, kind)
+        for name, attr in _GROUP_ATTR.items():
+            items.append((getattr(self, attr).detach(), kind_of.get(name, 0)))
+            st = self.optimizer.state.get(groups[name]["params"][0], None) if name in groups else None
+            if st is not None and "exp_avg" in st:
+                items += [(st["exp_avg"], 3), (st["exp_avg_sq"], 3)]
+        items += [(self.xyz_gradient_accum, 3), (self.denom, 3), (self.max_radii2D, 3)]
+        if getattr(self, "filter_3D", None) is not None:
+            items.append((self.filter_3D, 0))
+        if dev.type == "cuda":
+            for t, _ in items:
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev or t.shape[0] != P:
+                    raise _lib.DgsError("relocation rewrites the store in place: every per-Gaussian tensor must be a "
+                                        "contiguous float32 [P, ...] tensor on %s" % dev)
+            lib = _lib.load()
+            n, nt = int(dst.numel()), len(items)
+            dst_c, src_c = dst.to(torch.int64).contiguous(), src.to(torch.int64).contiguous()
+            scratch = torch.empty(int(lib.dgs_mcmc_relocate_scratch_bytes(n)), dtype=torch.uint8, device=dev)
+            with torch.cuda.device(dev):
+                rc = lib.dgs_mcmc_relocate(
+                    nt, (C.c_void_p * nt)(*[t.data_ptr() for t, _ in items]),
+                    (C.c_int * nt)(*[int(math.prod(t.shape[1:])) for t, _ in items]),
+                    (C.c_int * nt)(*[k for _, k in items]), n, _lib.ptr(dst_c), _lib.ptr(src_c), _lib.ptr(ratio),
+                    float(self.scale_lower_bound), int(bool(self.use_isotropic)), _lib.ptr(scratch),
+                    C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _lib.check(rc, "dgs_mcmc_relocate")
+        else:   # CPU tensors: the same plan with torch indexing, the values from the fp64 statement
+            op, sc, _, _ = mcmc.relocation_values(self._opacity.detach()[src], self._scaling.detach()[src], ratio,
+                                                  self.scale_lower_bound, self.use_isotropic)
+            for t, kind in items:
+                if kind == 0:
+                    t[dst] = t[src]
+                else:
+                    v = op if kind == 1 else sc if kind == 2 else 0.0
+                    t[dst] = v
+                    t[src] = v
+
+    @torch.no_grad()
+    def relocate_gs(self, dead_mask=None, min_opacity=0.005, generator=None):
+        """3DGS-MCMC relocation: every dead Gaussian (default: get_opacity <= min_opacity, the unfiltered getter) is
+        replaced, in place, by a copy of a live one drawn with probability proportional to its opacity
+        (mcmc.sample_by_opacity); the opacity and scale of each drawn source are split between it and its copies so
+        that the rendered image stays the same to first order.  Parameters, optimizer state, `filter_3D` and the
+        statistics keep their identity (a captured graph.BlurryViewGraph stays valid); the moments and statistics of
+        the touched rows are zeroed; step counts are kept.  Returns the number of rows relocated (0, doing nothing,
+        when no row is dead or none is live)."""
+        from . import mcmc
+        opac = self.get_opacity.detach().reshape(-1)
+        dead = (opac <= min_opacity) if dead_mask is None else dead_mask.reshape(-1).to(device=opac.device,
+                                                                                      dtype=torch.bool)
+        n_dead = int(dead.sum())
+        weights = torch.where(dead, torch.zeros_like(opac), opac)
+        if n_dead == 0 or float(torch.floor(weights.double().clamp(0.0, 1.0) * 2.0 ** 24).max()) <= 0.0:
+            return 0
+        dst = torch.nonzero(dead).squeeze(1)
+        src = mcmc.sample_by_opacity(weights, n_dead, generator)
+        self._relocate(dst, src)
+        return n_dead
+
+    @torch.no_grad()
+    def add_new_gs(self, cap_max, growth=0.05, generator=None):
+        """3DGS-MCMC growth: append min(cap_max, floor((1 + growth) P)) - P Gaussians, copies of rows drawn by opacity,
+        with the same opacity / scale split as `relocate_gs` (one `_rebuild` that appends the copies, then one
+        relocation whose destinations are the appended rows).  P changes: a captured graph must be rebuilt, as after
+        densify_and_prune.  Returns the number of rows added."""
+        from . import mcmc
+        P = self._xyz.shape[0]
+        n_new = mcmc.growth_target(P, cap_max, growth)
+        if n_new == 0:
+            return 0
+        src = mcmc.sample_by_opacity(self.get_opacity.detach(), n_new, generator)
+        self._rebuild(torch.cat((torch.arange(P, device=src.device), src)), P, keep_stats=True)
+        self._relocate(torch.arange(P, P + n_new, device=src.device), src)
+        return n_new
 
     @torch.no_grad()
     def reset_opacity(self, new_opacity=None):

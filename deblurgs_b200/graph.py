@@ -17,7 +17,7 @@ import torch
 
 from . import _lib
 from . import rasterizer as rz
-from .loss import photometric_loss
+from .loss import mcmc_regularization, photometric_loss
 
 
 class BlurryViewGraph:
@@ -32,13 +32,17 @@ class BlurryViewGraph:
     was changed raises DgsError (build a new BlurryViewGraph for the other setting) instead of rendering the old one.
     So is the 3-D filter (`filter_3D`): whether it is on and which tensor holds it are fixed at capture, and a replay
     after either changed raises.  Recomputing it in place (`CameraMotionModule.compute_3D_filter` on an unchanged
-    store) is what a replay sees: the graph reads the tensor's current values."""
+    store) is what a replay sees: the graph reads the tensor's current values.  The same holds for the in-place
+    3DGS-MCMC moves (`relocate_gs`, `mcmc.add_sgld_noise`); `add_new_gs` changes P and needs a new graph.
+    opacity_reg / scale_reg > 0 add loss.mcmc_regularization to the captured loss."""
 
     def __init__(self, cmm, cam_idx, background, gt_shape, lambda_t_smooth=0.0, parameters=None, pre_backward=None,
                  caller_owned_grads=(), capacity_margin=1.25, post_backward=None, render_fn=None,
-                 lambda_dssim=0.0):
+                 lambda_dssim=0.0, opacity_reg=0.0, scale_reg=0.0):
         self.cmm, self.cam_idx, self.bg, self.lam = cmm, cam_idx, background, float(lambda_t_smooth)
         self.lam_dssim = float(lambda_dssim)      # > 0: the D-SSIM term of loss.photometric_loss inside the graph
+        # 3DGS-MCMC's regularisers (loss.mcmc_regularization) inside the graph; both 0: not captured at all
+        self.opacity_reg, self.scale_reg = float(opacity_reg), float(scale_reg)
         dev = cmm.gaussians.get_xyz.device
         self.device = dev
         self.params = list(parameters) if parameters is not None else cmm.gaussians.parameters() + cmm.parameters()
@@ -70,6 +74,8 @@ class BlurryViewGraph:
         else:
             out = self.cmm.query(self.cam_idx, "all", background=self.bg)
         loss = photometric_loss(out["blurred"], out["subframes"], self.gt, self.lam, self.lam_dssim)
+        if self.opacity_reg != 0.0 or self.scale_reg != 0.0:
+            loss = loss + mcmc_regularization(self.cmm.gaussians, self.opacity_reg, self.scale_reg)
         loss.backward()
         if self.post_backward is not None:
             self.post_backward()

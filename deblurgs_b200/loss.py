@@ -211,6 +211,13 @@ def photometric_loss(blurred, subframes, gt, lambda_t_smooth=0.0, lambda_dssim=0
     return (1.0 - lam) * l1 + lam * (1.0 - ssim(blurred, gt.detach()))
 
 
+def mcmc_regularization(gaussians, opacity_reg=0.01, scale_reg=0.01):
+    """3DGS-MCMC's regularisers, opacity_reg * mean|get_opacity| + scale_reg * mean|get_scaling| (unfiltered getters):
+    they push unused Gaussians towards transparency, where relocation picks them up.  Two torch reductions,
+    differentiable in the raw opacity and scaling."""
+    return opacity_reg * gaussians.get_opacity.abs().mean() + scale_reg * gaussians.get_scaling.abs().mean()
+
+
 def training_loss(blurred, subframes, gt, depths=None, opacity=None, lambda_t_smooth=0.0, lambda_depth_tv=0.0,
                   lambda_hinge=0.0, lambda_dssim=0.0):
     """The reference's loss (train.py:147-163): Ll1 + lambda_t_smooth * L_t_smooth + lambda_depth_tv * L_depth_tv +

@@ -29,10 +29,13 @@ blending-weight sum is removed (prune_by_contribution); training then continues 
 training view after initialisation, every --filter3d-every iterations and after each densify round.  The views are
 also scored at double size (a camera of 2W x 2H with the same field of view, against the hidden scene rendered sharp
 at that size without the filter): the zoom-in case the filter is for.
+--mcmc: 3DGS-MCMC densification instead of densify_and_prune: every --densify-every iterations the dead Gaussians
+(opacity <= 0.005) are relocated onto live ones and the store grows by 5 % up to --cap-max (default 2x --gaussians);
+SGLD position noise after every optimizer step and the opacity / scale regularisers (0.01 each) in the loss.
 
   python examples/train_blurry_views.py [--iters 200] [--views 4] [--gaussians 20000] [--lambda-dssim 0.2]
                                         [--antialiasing] [--prune-fraction 0.5 [--prune-at 100]]
-                                        [--filter3d [--filter3d-every 100]]
+                                        [--filter3d [--filter3d-every 100]] [--mcmc [--cap-max N]]
 """
 import argparse
 import os
@@ -43,7 +46,8 @@ import types
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from deblurgs_b200 import renderer, synthetic, training_loss  # noqa: E402
+from deblurgs_b200 import mcmc, renderer, synthetic, training_loss  # noqa: E402
+from deblurgs_b200.loss import mcmc_regularization  # noqa: E402
 from deblurgs_b200.motion import CameraMotionModule, GaussianParams  # noqa: E402
 from deblurgs_b200.pose import bezier_se3_poses  # noqa: E402
 from deblurgs_b200.refine import evaluate_views  # noqa: E402
@@ -85,7 +89,12 @@ def main():
     ap.add_argument("--prune-at", type=int, default=None, help="iteration of the contribution pruning (default iters/2)")
     ap.add_argument("--filter3d", action="store_true", help="3-D smoothing filter on the trained store (Mip-Splatting)")
     ap.add_argument("--filter3d-every", type=int, default=100, help="recompute the 3-D filter every N iterations")
+    ap.add_argument("--mcmc", action="store_true", help="3DGS-MCMC relocation / growth / SGLD noise instead of "
+                    "densify_and_prune")
+    ap.add_argument("--cap-max", type=int, default=None, help="--mcmc: Gaussian budget (default 2x --gaussians)")
     args = ap.parse_args()
+    cap_max = 2 * args.gaussians if args.cap_max is None else args.cap_max
+    mcmc_gen = torch.Generator().manual_seed(7)
     prune_at = args.iters // 2 if args.prune_at is None else args.prune_at
     if args.width % 2 or args.height % 2:
         raise SystemExit("--width and --height must be even (the half-resolution views average 2x2 pixel boxes)")
@@ -169,12 +178,24 @@ def main():
         out = cmm.query(idx, "all", background=bg)
         loss = training_loss(out["blurred"], out["subframes"], out["gt"], lambda_t_smooth=lam,
                              lambda_dssim=args.lambda_dssim)
+        if args.mcmc:
+            loss = loss + mcmc_regularization(gauss)
         loss.backward()
         with torch.no_grad():
             gauss.add_densification_stats_blurry(out["batched"])    # train.py:188-193, from the backward's epilogue
         opt.step(clip_grad_value=1.0)
         opt.zero_grad(set_to_none=True)
-        if args.densify_every and it > 0 and it % args.densify_every == 0 and it < args.iters - 1:
+        if args.mcmc:
+            mcmc.add_sgld_noise(gauss, opt.param_groups[0]["lr"], it)
+        if args.mcmc and args.densify_every and it > 0 and it % args.densify_every == 0 and it < args.iters - 1:
+            n_before = gauss.get_xyz.shape[0]
+            n_moved = gauss.relocate_gs(generator=mcmc_gen)
+            n_added = gauss.add_new_gs(cap_max, generator=mcmc_gen)
+            print("iter %4d  MCMC: %d relocated, %d added: %d -> %d Gaussians (cap %d)"
+                  % (it, n_moved, n_added, n_before, gauss.get_xyz.shape[0], cap_max), flush=True)
+            if args.filter3d and n_added:
+                cmm.compute_3D_filter()
+        elif args.densify_every and it > 0 and it % args.densify_every == 0 and it < args.iters - 1:
             n_before = gauss.get_xyz.shape[0]
             gauss.densify_and_prune(max_grad=2e-4, extent=5.0)       # train.py:195-196
             print("iter %4d  densify/prune: %d -> %d Gaussians" % (it, n_before, gauss.get_xyz.shape[0]), flush=True)

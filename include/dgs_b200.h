@@ -493,6 +493,50 @@ int dgs_adam_step(int n_tensors, float* const* params, const float* const* grads
 int dgs_rows_gather(int n_tensors, const float* const* in, float* const* out, const int* width, const int* zero_new,
                     int64_t n_out, const int64_t* src_rows, const uint8_t* carry, void* stream);
 
+/*
+ * 3DGS-MCMC densification (Kheradmand et al., NeurIPS 2024) on the parameter store, in place.
+ *
+ * dgs_mcmc_relocate moves n Gaussians: entry r copies source row src_rows[r] into destination row dst_rows[r] and
+ * splits the source's opacity and scale between the 1 + (copies) Gaussians that now share it, keeping the rendered
+ * image unchanged to first order.  ratio[r] = N = 1 + (number of entries with the same source), clamped to [1, 51]:
+ *   o  = clamp(opacity[src], 0, 1)                 (the raw opacity is the activated one: the activation is a clamp)
+ *   o' = 1 - (1 - o)^(1/N), stored clamped to [0.005, 1 - 2^-23] (the lower bound is the smallest float above 0.005:
+ *        a relocated Gaussian never counts as dead by the rule opacity <= 0.005); c uses the unclamped o'
+ *   c  = o / D(o', N),  D = sum_{j=1..N} (-1)^(j-1) C(N,j) o'^j / sqrt(j)   (fp64; equal to the paper's double sum)
+ *   raw scaling' = raw + log(c) when scale_lower_bound == 0, else log(max(c (exp(raw) + lb) - lb, 0.001));
+ *   isotropic != 0: every column from column 0, as get_scaling expands it.
+ * HOST arrays of n_tensors (<= DGS_GATHER_MAX_TENSORS) entries: device pointers `tensors` (fp32, [P, width[k]],
+ * rewritten in place), width[k] and kind[k]:
+ *   DGS_RELOCATE_COPY     dst row <- src row                    (xyz, features, rotation, the 3-D filter)
+ *   DGS_RELOCATE_OPACITY  dst and src rows <- o'                (exactly one, width 1)
+ *   DGS_RELOCATE_SCALING  dst and src rows <- raw scaling'      (exactly one, width 3)
+ *   DGS_RELOCATE_ZERO     dst and src rows <- 0                 (Adam moments, densification statistics)
+ * dst_rows, src_rows [n] int64 and ratio [n] int32 on the device.  PRECONDITION: the destination rows are distinct
+ * and no destination row is a source row (sources are drawn from live Gaussians, destinations are dead or appended
+ * ones); entries sharing a source must carry the same ratio.  scratch: dgs_mcmc_relocate_scratch_bytes(n) bytes,
+ * 16-B aligned.  Two launches, no allocation, no host synchronisation.
+ *
+ * dgs_mcmc_noise: the SGLD step after the optimizer, for every Gaussian g < P:
+ *   xyz[g] += Sigma eps gate step_scale,  Sigma = R diag(s^2) R^T,  gate = 1 / (1 + exp(-k ((1 - clamp(o,0,1)) - x0)))
+ * with s = exp(scaling) + scale_lower_bound (isotropic: column 0), R the rotation of the normalised quaternion
+ * (w, x, y, z; norm floored at 1e-12) and eps ~ N(0, I3) drawn in the kernel: Philox4x32-10 with key seed (low word
+ * first) and counter (g, step) (low words first), then Box-Muller on the pairs (x0, x1) and (x2, x3) of its output, the
+ * uniforms being ((x >> 8) + 0.5) / 2^24.  eps is a pure function of (seed, step, g).
+ * dgs_debug_mcmc_normals writes that eps to out [P, 3] (test hook).
+ */
+#define DGS_RELOCATE_COPY 0
+#define DGS_RELOCATE_OPACITY 1
+#define DGS_RELOCATE_SCALING 2
+#define DGS_RELOCATE_ZERO 3
+size_t dgs_mcmc_relocate_scratch_bytes(int64_t n);
+int dgs_mcmc_relocate(int n_tensors, float* const* tensors, const int* width, const int* kind, int64_t n,
+                      const int64_t* dst_rows, const int64_t* src_rows, const int32_t* ratio, float scale_lower_bound,
+                      int isotropic, void* scratch, void* stream);
+int dgs_mcmc_noise(int64_t P, float* xyz, const float* scaling, const float* rotation, const float* opacity,
+                   float scale_lower_bound, int isotropic, float step_scale, float k, float x0, uint64_t seed,
+                   int64_t step, void* stream);
+int dgs_debug_mcmc_normals(int64_t P, uint64_t seed, int64_t step, float* out, void* stream);
+
 /* present [P] uint8: 1 iff view-space z > 0.2 (reference in_frustum, auxiliary.h:144-169). */
 int dgs_mark_visible(int P, const float* means3D, const float* viewmatrix,
                      const float* projmatrix, uint8_t* present, void* stream);
